@@ -2,6 +2,7 @@
 """Benchmark of the YOLO-Fastest detection hot path (forward + decode + confidence filter + per-class NMS).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--res 512x640|256x320] [--batch B]
+                    [--dump-outputs DIR]
 
 One step = one pass of the hot path over one batch of synthetic images per GPU.  Default workload
 (BASELINE.json metric): 640x512 images, batch 256 per GPU, the shipped 512x640 checkpoint.  Weak scaling:
@@ -17,6 +18,9 @@ Prints ONE JSON line on rank 0:
   cpu_baseline  the oracle port of the reference (PyTorch CPU forward + the reference's Python decode/NMS loops)
                 timed on this box's host cores on a bounded sample (rank 0, N=1 only)
 --impl reference times that CPU port alone, with all host threads, on the same workload definition.
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0) as float64 .npy files (dump_outputs), so that
+two builds can be compared output for output: the inputs are seeded and the same from run to run.
+The benchmark writes nothing into the tree (it may be read-only): no bytecode caches, and build() leaves current libraries alone.
 """
 import argparse
 import json
@@ -134,6 +138,33 @@ def synthetic_u8(B, H, W, seed):
     return torch.randint(0, 256, (B, H, W), generator=g, dtype=torch.uint8)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(d, out, counts, status):
+    """What Detect_YOLO.detect_device returned for one batch, as float64 arrays under d:
+      detections.npy  [N, max_det, 8]  x1, y1, x2, y2, conf, cls_score, cls, src of each record of the slab; the slots after an
+                                       image's min(count, max_det) records hold no record (unset memory) and are written as 0
+      counts.npy      [N]              untruncated detection count of each image
+      status.npy      [N]              status word of each image
+      image_index.npy [N]              which images of the batch these are: all of them, or a fixed seeded sample when the
+                                       arrays of the whole batch would exceed DUMP_LIMIT_BYTES"""
+    from yolo_fastest_b200 import _lib
+    B, max_det = out.shape[0], out.shape[1]
+    recs = out.cpu().numpy().view(_lib.DET_DTYPE).reshape(B, max_det)
+    cnt, st = counts.cpu().numpy(), status.cpu().numpy()
+    per_image = 8 * (max_det * 8 + 3)
+    idx = np.arange(B)
+    if B * per_image > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(B, DUMP_LIMIT_BYTES // per_image, replace=False))
+    recs, cnt, st = recs[idx], cnt[idx], st[idx]
+    dets = np.stack([recs[f].astype(np.float64) for f in _lib.DET_DTYPE.names], axis=-1)
+    dets[np.arange(max_det)[None, :] >= np.minimum(cnt, max_det)[:, None]] = 0.0
+    os.makedirs(d, exist_ok=True)
+    for name, a in (("detections", dets), ("counts", cnt), ("status", st), ("image_index", idx)):
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def cpu_reference_pass(sd, io, u8, res):
     """One pass of the reference's CPU path over a batch: (forward s, post-process s, detections, kind).
     kind "reference": the UNMODIFIED reference staged under baseline/_ref (baseline/ref_arm.py: its own YoloFastest module and
@@ -210,7 +241,11 @@ def main():
                     help="images per CPU-baseline pass: a bounded sample of the batch-256 workload, at the batch size the host runs fastest "
                          "(measured on the GPU box's 16 cores: 50 img/s at 16 images per pass, 43 img/s at 32)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the detections of the last timed step as .npy files under DIR (rank 0; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3                                     # timing rules: W >= 3
 
@@ -273,7 +308,7 @@ def main():
         out, counts, status = det.detect_device(x_dev, args.max_det)
         if world > 1:
             gather_compact(out, counts, n_total, dst=0, ctx=det.model._ctx)   # compaction kernel + one NCCL gather on the side stream
-        return counts
+        return out, counts, status
 
     def step_e2e():
         rows = det.detect_batch(u8, max_det=args.max_det, raw=True)
@@ -292,7 +327,7 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        counts = step_device()
+        last = step_device()
     e1.record()
     torch.cuda.synchronize(dev)
     ms = e0.elapsed_time(e1)
@@ -303,7 +338,9 @@ def main():
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
-    n_det = int(counts.sum().item())
+    n_det = int(last[1].sum().item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
 
     # ---- end to end through the public API with host buffers ------------------------------------------------
     # serving loop on the double-buffered API: batch i+1 is submitted (H2D copy on the copy stream) before the
@@ -536,4 +573,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True          # the project modules main() imports leave no __pycache__ in the tree
     main()
