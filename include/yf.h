@@ -216,6 +216,24 @@ int yf_preprocess_bgr(yf_ctx* ctx, const uint8_t* bgr, int B, int Ho, int Wo, ui
 int yf_detect_host_bgr(yf_ctx* ctx, const uint8_t* bgr_host, int B, int Ho, int Wo, const yf_post_params* p,
                        yf_det* out_host, int32_t* counts_host, int32_t* status_host, void* stream);
 
+/* The same for a batch whose frames may differ in size, and for colour networks: frames dev holds B BGR uint8 frames back to back,
+ * frame b at byte offset off[b] with shape [Ho[b], Wo[b], 3] and contiguous rows, 1 <= Ho[b], Wo[b] <= 16384. off / Ho / Wo are
+ * HOST arrays, B <= max_batch. out dev: [B, H, W] gray when in_ch == 1 (the bytes of yf_preprocess_bgr), [B, 3, H, W] R, G, B planes
+ * when in_ch == 3 (detect.py:107-122 for a colour network: cv2.resize of the BGR frame, then [:, :, ::-1] and HWC -> CHW; the 11-bit
+ * arithmetic of the gray path once per channel). The coefficients are computed on the device for each frame, so sizes may change from
+ * call to call, and within a call, without a synchronisation. Frames whose rows are 4-byte aligned (width a multiple of 4, aligned
+ * offset) are read fastest; any layout works. Bad descriptors fail with YF_ERR_ARG before anything is enqueued. */
+int yf_preprocess_frames(yf_ctx* ctx, const uint8_t* frames, int B, const int64_t* off, const int32_t* Ho, const int32_t* Wo,
+                         uint8_t* out, void* stream);
+
+/* yf_detect_host_bgr for such a batch: frames_host holds the packed frames in `nbytes` bytes of HOST memory (pinned for an
+ * asynchronous copy; every descriptor must lie inside them). One copy of the nbytes to the device, yf_preprocess_frames, yf_detect,
+ * and the results back as yf_detect_host_u8 returns them, in NETWORK-input coordinates (scaling back to each frame stays with the
+ * caller). Synchronises `stream`. */
+int yf_detect_host_frames(yf_ctx* ctx, const uint8_t* frames_host, int64_t nbytes, int B, const int64_t* off, const int32_t* Ho,
+                          const int32_t* Wo, const yf_post_params* p, yf_det* out_host, int32_t* counts_host,
+                          int32_t* status_host, void* stream);
+
 /* ---- introspection ---------------------------------------------------------------------- */
 
 /* Kernels launched by this ctx since creation (the bench's gpu_launches evidence). */

@@ -61,6 +61,8 @@ SYMBOLS = [
     ("yf_detect_submit_u8_dev", C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(YfPostParams), _P, _P, _P]),
     ("yf_preprocess_bgr", C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P, _P]),
     ("yf_detect_host_bgr", C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.POINTER(YfPostParams), _P, _P, _P, _P]),
+    ("yf_preprocess_frames", C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P, _P]),
+    ("yf_detect_host_frames", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.POINTER(YfPostParams), _P, _P, _P, _P]),
     ("yf_compact_dets", C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P]),
     ("yf_launch_count", C.c_int64, [_P]),
     ("yf_profile_forward", C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.c_int]),

@@ -207,7 +207,8 @@ struct yf_ctx {
     bool sl_used[2] = {false, false};
     // CUDA graphs of forward + head kernel on the library's own fixed buffers (small batches: launch latency dominates)
     std::map<std::string, std::pair<cudaGraphExec_t, int>> graphs;    // key -> (executable graph, kernel launches inside)
-    // GPU pre-processing (yf_preprocess_bgr / yf_detect_host_bgr): coefficient tables of the last source size, BGR staging
+    // GPU pre-processing (yf_preprocess_bgr / yf_detect_host_bgr): coefficient tables of the last source size; BGR staging (also of
+    // yf_detect_host_frames, whose kernel computes its taps itself)
     PrepTap* prep_tab = nullptr;                        // [W column taps | H row taps]
     int prep_Ho = 0, prep_Wo = 0;
     unsigned char* d_bgr = nullptr;
@@ -1411,6 +1412,8 @@ extern "C" int yf_create_variant(yf_ctx** out, int device, int in_ch, int num_cl
         cudaFuncSetAttribute(post_kernel<YF_MODE_DETECT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 12),
         cudaFuncSetAttribute(post_kernel<YF_MODE_VALIDATE>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 12),
         cudaFuncSetAttribute(post_kernel<POST_SRC_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 12),
+        cudaFuncSetAttribute(prep_frames_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
+        cudaFuncSetAttribute(prep_frames_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
         init_irb<CfgRes2>(), init_irb<CfgDown2>(), init_irb<CfgRes3a>(), init_irb<CfgWide3>(),
         init_irb<CfgRes3b>(), init_irbtc<CfgRes3bTc>(), init_irbt<CfgRes3bTt>(), init_irbt<CfgRes4Tt>(), init_irbt<CfgRes3aTt>(), init_irbt<CfgWide3Tt>(), init_irbt<CfgDown3Tt>(), init_irbt<CfgDown4Tt>(), init_irbtc<CfgRes4Tc>(), init_irbtc2<CfgRes5Tc>(), init_irbtc2<CfgRes5TcS>(), init_irbtc2<CfgRes5TcXS>(), init_irbtc2<CfgRes5TcN>(), init_dwpwtc<CfgNeckS1TcS>(), init_dwpwtc<CfgNeckS2TcS>(), init_irbtc<CfgRes3bTcXS>(), init_irbtc<CfgRes4TcXS>(), init_dwpwtc<CfgNeckS1TcN>(), init_dwpwtc<CfgNeckS2TcN>(), init_dwpwtc<CfgNeckL1TcN>(), init_dwpwtc<CfgNeckL2TcN>(), init_irb<CfgDown3N>(), init_irb<CfgDown4N>(), init_dwpwtc<CfgNeckL1TcS>(), init_dwpwtc<CfgNeckL2TcS>(), init_irbtc<CfgRes3bTcS>(), init_irbtc<CfgRes4TcS>(), init_dwpwtc<CfgNeckS1Tc>(), init_dwpwtc<CfgNeckL1Tc>(), init_dwpwtc<CfgNeckS2Tc>(), init_dwpwtc<CfgNeckL2Tc>(), init_irb<CfgDown3>(), init_irb<CfgRes4>(), init_irb<CfgDown4>(), init_irb<CfgRes5>(),
         init_irb<CfgNeckS1>(), init_irb<CfgNeckS2>(), init_irb<CfgNeckL1>(), init_irb<CfgNeckL2>()};
@@ -1925,6 +1928,17 @@ static int prep_enqueue(yf_ctx* ctx, const uint8_t* bgr_dev, int B, int Ho, int 
     return YF_OK;
 }
 
+// grow-only device staging of host frames (yf_detect_host_bgr / yf_detect_host_frames)
+static int ensure_bgr(yf_ctx* ctx, size_t nbytes, cudaStream_t st) {
+    if (nbytes <= ctx->bgr_cap) return YF_OK;
+    CU(cudaStreamSynchronize(st));                      // an earlier call's kernels may still read the old buffer
+    if (ctx->d_bgr) CU(cudaFree(ctx->d_bgr));
+    ctx->d_bgr = nullptr; ctx->bgr_cap = 0;
+    CU(cudaMalloc(&ctx->d_bgr, nbytes));
+    ctx->bgr_cap = nbytes;
+    return YF_OK;
+}
+
 extern "C" int yf_preprocess_bgr(yf_ctx* ctx, const uint8_t* bgr_dev, int B, int Ho, int Wo, uint8_t* gray_dev, void* stream) {
     CTX_CHECK(ctx);
     if (!bgr_dev || !gray_dev || B < 1) { set_err(&ctx->err, "bad argument"); return YF_ERR_ARG; }
@@ -1945,18 +1959,91 @@ extern "C" int yf_detect_host_bgr(yf_ctx* ctx, const uint8_t* bgr_host, int B, i
     int rc = ensure_out(ctx, p->max_det);
     if (rc) return rc;
     const size_t nbytes = (size_t)B * Ho * Wo * 3;
-    if (nbytes > ctx->bgr_cap) {
-        CU(cudaStreamSynchronize(st));
-        if (ctx->d_bgr) CU(cudaFree(ctx->d_bgr));
-        ctx->d_bgr = nullptr; ctx->bgr_cap = 0;
-        CU(cudaMalloc(&ctx->d_bgr, nbytes));
-        ctx->bgr_cap = nbytes;
-    }
+    if ((rc = ensure_bgr(ctx, nbytes, st))) return rc;
     CU(cudaMemcpyAsync(ctx->d_bgr, bgr_host, nbytes, cudaMemcpyHostToDevice, st));
     rc = prep_enqueue(ctx, ctx->d_bgr, B, Ho, Wo, ctx->d_u8, st);
     if (rc) return rc;
     rc = detect_fixed(ctx, ctx->d_u8, true, B, p, ctx->d_out, ctx->d_counts, ctx->d_status, st);
     if (rc) return rc;
+    CU(cudaMemcpyAsync(out_host, ctx->d_out, sizeof(yf_det) * (size_t)B * p->max_det, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(counts_host, ctx->d_counts, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    if (status_host) CU(cudaMemcpyAsync(status_host, ctx->d_status, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return YF_OK;
+}
+
+// ---- frames of mixed sizes, gray or colour networks (one launch per PREP_CHUNK frames, taps computed in the kernel) --------------
+static const int kPrepMaxSide = 16384;
+
+// every descriptor against the size range and, when the buffer size is known (nbytes >= 0), against the buffer
+static int frames_check(yf_ctx* ctx, int B, const int64_t* off, const int32_t* Ho, const int32_t* Wo, int64_t nbytes) {
+    if (!off || !Ho || !Wo) { set_err(&ctx->err, "null descriptor array"); return YF_ERR_ARG; }
+    if (B < 1 || B > ctx->max_batch) { set_err(&ctx->err, "batch %d outside [1, max_batch=%d]", B, ctx->max_batch); return YF_ERR_ARG; }
+    for (int b = 0; b < B; ++b) {
+        if (Ho[b] < 1 || Wo[b] < 1 || Ho[b] > kPrepMaxSide || Wo[b] > kPrepMaxSide) {
+            set_err(&ctx->err, "frame %d: size %dx%d outside [1, %d]", b, Ho[b], Wo[b], kPrepMaxSide); return YF_ERR_ARG;
+        }
+        const int64_t size = (int64_t)Ho[b] * Wo[b] * 3;
+        if (off[b] < 0 || (nbytes >= 0 && off[b] > nbytes - size)) {
+            set_err(&ctx->err, "frame %d: bytes [%lld, %lld) outside the %lld-byte buffer", b, (long long)off[b], (long long)(off[b] + size),
+                    (long long)nbytes);
+            return YF_ERR_ARG;
+        }
+    }
+    return YF_OK;
+}
+
+static int frames_enqueue(yf_ctx* ctx, const uint8_t* frames, int B, const int64_t* off, const int32_t* Ho, const int32_t* Wo,
+                          uint8_t* out, cudaStream_t st) {
+    const int nsm = ctx->groups.empty() ? 148 : ctx->groups[0].a.nsm;
+    const long long groups = (ctx->H + PREP_R - 1) / PREP_R;
+    const size_t per_img = (size_t)ctx->in_ch * ctx->H * ctx->W;
+    PrepFrames fr;
+    for (int c0 = 0; c0 < B; c0 += PREP_CHUNK) {
+        const int n = std::min(PREP_CHUNK, B - c0);
+        int smem = 0;                                   // from the widest frame of the chunk that is staged
+        for (int i = 0; i < n; ++i) {
+            fr.f[i] = {off[c0 + i], Ho[c0 + i], Wo[c0 + i]};
+            if (prep_stageable(frames, fr.f[i], ctx->in_ch, PREP_SMEM_CAP)) smem = std::max(smem, prep_stage_bytes(fr.f[i].Wo, ctx->in_ch));
+        }
+        auto kern = ctx->in_ch == 1 ? prep_frames_kernel<1> : prep_frames_kernel<3>;
+        int per_sm = 1;                                 // resident blocks: the grid strides over the rest
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, PREP_NT, smem));
+        const int grid = (int)std::min<long long>((long long)n * groups, (long long)nsm * std::max(per_sm, 1));
+        kern<<<grid, PREP_NT, smem, st>>>(frames, fr, n, out + c0 * per_img, ctx->H, ctx->W, smem);
+        CU(cudaGetLastError());
+        ctx->launches += 1;
+    }
+    return YF_OK;
+}
+
+extern "C" int yf_preprocess_frames(yf_ctx* ctx, const uint8_t* frames, int B, const int64_t* off, const int32_t* Ho, const int32_t* Wo,
+                                    uint8_t* out, void* stream) {
+    CTX_CHECK(ctx);
+    if (!frames || !out) { set_err(&ctx->err, "null frames or output pointer"); return YF_ERR_ARG; }
+    int rc = frames_check(ctx, B, off, Ho, Wo, -1);
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    return frames_enqueue(ctx, frames, B, off, Ho, Wo, out, (cudaStream_t)stream);
+}
+
+extern "C" int yf_detect_host_frames(yf_ctx* ctx, const uint8_t* frames_host, int64_t nbytes, int B, const int64_t* off, const int32_t* Ho,
+                                     const int32_t* Wo, const yf_post_params* p, yf_det* out_host, int32_t* counts_host,
+                                     int32_t* status_host, void* stream) {
+    CTX_CHECK(ctx);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!frames_host || !p || !out_host || !counts_host) { set_err(&ctx->err, "null argument"); return YF_ERR_ARG; }
+    if (p->max_det < 1) { set_err(&ctx->err, "max_det must be >= 1"); return YF_ERR_ARG; }
+    int rc = frames_check(ctx, B, off, Ho, Wo, nbytes);
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    if (!ctx->weights_loaded) { set_err(&ctx->err, "yf_load_weights has not been called"); return YF_ERR_STATE; }
+    ORDER(ctx, st);
+    if ((rc = ensure_out(ctx, p->max_det))) return rc;
+    if ((rc = ensure_bgr(ctx, (size_t)nbytes, st))) return rc;
+    CU(cudaMemcpyAsync(ctx->d_bgr, frames_host, (size_t)nbytes, cudaMemcpyHostToDevice, st));      // the packed frames, one copy
+    if ((rc = frames_enqueue(ctx, ctx->d_bgr, B, off, Ho, Wo, ctx->d_u8, st))) return rc;
+    if ((rc = detect_fixed(ctx, ctx->d_u8, true, B, p, ctx->d_out, ctx->d_counts, ctx->d_status, st))) return rc;
     CU(cudaMemcpyAsync(out_host, ctx->d_out, sizeof(yf_det) * (size_t)B * p->max_det, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(counts_host, ctx->d_counts, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
     if (status_host) CU(cudaMemcpyAsync(status_host, ctx->d_status, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));

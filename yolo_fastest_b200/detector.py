@@ -178,6 +178,44 @@ def _check_u8_host(t, input_shape, what):
         raise _lib.YfError("%s serves the single-channel networks" % what)
 
 
+FRAME_ALIGN = 16          # byte alignment of every packed frame (32-bit row loads in the pre-processing kernel need 4)
+MAX_FRAME_SIDE = 16384
+
+
+def frame_layout(frames):
+    """Validate a list of BGR uint8 frames [h, w, 3] (numpy arrays or torch tensors, sizes may differ) and lay them out back to back:
+    -> (off int64 [B], Ho int32 [B], Wo int32 [B], nbytes), frame b at byte offset off[b], every offset a multiple of FRAME_ALIGN."""
+    if not isinstance(frames, (list, tuple)) or len(frames) == 0:
+        raise _lib.YfError("frames: a non-empty list of uint8 BGR frames [h, w, 3]")
+    B = len(frames)
+    off, Ho, Wo = np.zeros(B, np.int64), np.zeros(B, np.int32), np.zeros(B, np.int32)
+    pos = 0
+    for b, f in enumerate(frames):
+        if isinstance(f, torch.Tensor):
+            u8 = f.dtype == torch.uint8
+        elif isinstance(f, np.ndarray):
+            u8 = f.dtype == np.uint8
+        else:
+            raise _lib.YfError("frame %d is a %s, not a numpy array or torch tensor" % (b, type(f).__name__))
+        if not u8:
+            raise _lib.YfError("frame %d is %s, frames are uint8" % (b, f.dtype))
+        if f.ndim != 3 or f.shape[2] != 3:
+            raise _lib.YfError("frame %d has shape %s, frames are BGR [h, w, 3]" % (b, tuple(f.shape)))
+        h, w = int(f.shape[0]), int(f.shape[1])
+        if not (1 <= h <= MAX_FRAME_SIDE and 1 <= w <= MAX_FRAME_SIDE):
+            raise _lib.YfError("frame %d is %dx%d, sizes must lie in [1, %d]" % (b, h, w, MAX_FRAME_SIDE))
+        off[b], Ho[b], Wo[b] = pos, h, w
+        pos += -(-h * w * 3 // FRAME_ALIGN) * FRAME_ALIGN
+    return off, Ho, Wo, int(off[-1]) + int(Ho[-1]) * int(Wo[-1]) * 3
+
+
+def pack_frames(frames, dst, off):
+    """Copy host frames into the uint8 numpy buffer `dst` at the offsets of frame_layout (any strides)."""
+    for f, o in zip(frames, off):
+        a = f.numpy() if isinstance(f, torch.Tensor) else f
+        dst[int(o):int(o) + a.size].reshape(a.shape)[...] = a
+
+
 class Detect_YOLO:
     def __init__(self, device, model_path, config_params, logger):
         device = torch.device(device)
@@ -201,6 +239,8 @@ class Detect_YOLO:
         self.colors = [[106, 90, 205], [199, 97, 20], [112, 128, 105]]
         self._pinned = {}
         self._slots = {}
+        self._frames_pin = None        # grow-only pinned staging of packed host frames (pre_process_frames / detect_frames)
+        self._frames_ev = None         # end of the last asynchronous copy out of it
 
     # ---- host-side image handling (unchanged semantics, detect.py:107-139) ------------------------
     def _load_gray(self, img_path):
@@ -283,6 +323,84 @@ class Detect_YOLO:
         if adjust and [Ho, Wo] != [H, W]:
             scale_h, scale_w = Ho / H, Wo / W
             for rr in rows:
+                for r in rr:
+                    r[0] = round(r[0] * scale_w)
+                    r[2] = round(r[2] * scale_w)
+                    r[1] = round(r[1] * scale_h)
+                    r[3] = round(r[3] * scale_h)
+        return rows
+
+    # ---- frames of mixed sizes, gray or colour networks (yf_preprocess_frames / yf_detect_host_frames) --------------------------
+    def _frames_pinned(self, nbytes):
+        if self._frames_ev is not None:
+            self._frames_ev.synchronize()           # the previous copy out of the buffer has finished before it is rewritten
+            self._frames_ev = None
+        if self._frames_pin is None or self._frames_pin.numel() < nbytes:
+            self._frames_pin = None
+            self._frames_pin = torch.empty((nbytes,), dtype=torch.uint8).pin_memory()
+        return self._frames_pin
+
+    def pre_process_frames(self, frames):
+        """A list of BGR uint8 frames [h_i, w_i, 3] as cv2.imread returns them, sizes free (all numpy / host torch, or all cuda
+        tensors) -> cuda uint8 [B, H, W] gray for single-channel networks, [B, 3, H, W] R, G, B planes for 3-channel ones: the
+        image half of detect.py:107-122 for each frame, byte-identical to OpenCV, in one kernel launch per 512 frames. Host frames
+        are packed into a pinned buffer and copied once; cuda frames are packed on the device."""
+        off, Ho, Wo, nbytes = frame_layout(frames)
+        on_dev = [isinstance(f, torch.Tensor) and f.is_cuda for f in frames]
+        if any(on_dev) and not all(on_dev):
+            raise _lib.YfError("pre_process_frames: frames must be all on the host or all on the device")
+        B = len(frames)
+        H, W, chans = self.input_shape[0:3]
+        ctx = self.model.context(self.device, H, W, B)
+        out = torch.empty((B, H, W) if chans == 1 else (B, chans, H, W), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device)
+            packed = torch.empty((nbytes,), dtype=torch.uint8, device=self.device)
+            if all(on_dev):
+                for f, o in zip(frames, off):
+                    packed[int(o):int(o) + f.numel()].view(f.shape).copy_(f)
+            else:
+                pin = self._frames_pinned(nbytes)
+                pack_frames(frames, pin.numpy(), off)
+                packed.copy_(pin[:nbytes], non_blocking=True)
+                self._frames_ev = torch.cuda.Event()
+                self._frames_ev.record(stream)
+            _lib.check(_lib.lib().yf_preprocess_frames(ctx.handle, packed.data_ptr(), B, off.ctypes.data, Ho.ctypes.data, Wo.ctypes.data,
+                                                      out.data_ptr(), C.c_void_p(stream.cuda_stream)), ctx.handle)
+        return out
+
+    def detect_frames(self, frames, max_det=64, raw=False, adjust=True):
+        """Host BGR uint8 frames [h_i, w_i, 3] of any sizes (a list) -> per-image rows: one yf_detect_host_frames call (one copy of
+        the packed frames, pre-processing, forward, decode, NMS, the result slab back), for gray and colour networks alike.
+        With adjust=True each frame's boxes are mapped back to THAT frame's size with the arithmetic of adjust_coord
+        (round(v * (h_i / H)), round(v * (w_i / W)); detect.py:131-139), which is batch_detect's result for a frame of
+        origin_img_shape."""
+        off, Ho, Wo, nbytes = frame_layout(frames)
+        if any(isinstance(f, torch.Tensor) and f.is_cuda for f in frames):
+            raise _lib.YfError("detect_frames takes host frames (pre_process_frames serves cuda frames)")
+        B = len(frames)
+        H, W = self.input_shape[0:2]
+        ctx = self.model.context(self.device, H, W, B)
+        pin = self._frames_pinned(nbytes)
+        pack_frames(frames, pin.numpy(), off)
+        pin_out = torch.empty((B, max_det, _lib.DET_DTYPE.itemsize), dtype=torch.uint8).pin_memory()
+        pin_cnt = torch.empty((B,), dtype=torch.int32).pin_memory()
+        pin_st = torch.empty((B,), dtype=torch.int32).pin_memory()
+        p = self.post_process._params(_lib.MODE_DETECT, max_det)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().yf_detect_host_frames(ctx.handle, pin.data_ptr(), nbytes, B, off.ctypes.data, Ho.ctypes.data,
+                                                       Wo.ctypes.data, C.byref(p), pin_out.data_ptr(), pin_cnt.data_ptr(),
+                                                       pin_st.data_ptr(), C.c_void_p(stream)), ctx.handle)
+        res = _finish(pin_out, pin_cnt, pin_st, B, max_det, lambda need: self.detect_frames(frames, max_det=need, raw=True, adjust=False))
+        if raw:
+            return res
+        rows = [_rows_from_dets(d) for d in res]
+        if adjust:
+            for rr, h, w in zip(rows, Ho, Wo):
+                if [int(h), int(w)] == [H, W]:
+                    continue
+                scale_h, scale_w = int(h) / H, int(w) / W
                 for r in rr:
                     r[0] = round(r[0] * scale_w)
                     r[2] = round(r[2] * scale_w)
@@ -448,7 +566,8 @@ class Detect_YOLO:
         """batch_detect with the per-file loop turned into batches (SURVEY 8f-1): the frames of `batch_size` files are
         decoded on the host (cv2.imread), everything else - gray, resize, normalisation, forward, decode, NMS - is ONE
         yf_detect_host_bgr call per batch. Same result files and log lines as batch_detect (detect.py:141-192); the two
-        per-image times of the log line are the batch's time divided by its size. Frames of one batch must share a size."""
+        per-image times of the log line are the batch's time divided by its size. A batch whose frames differ in size, or any batch
+        of a 3-channel network, goes through detect_frames instead (boxes scaled to each frame's own size)."""
         import cv2
         img_list = os.listdir(data_path)
         num = len(img_list)
@@ -458,7 +577,10 @@ class Detect_YOLO:
             frames = [cv2.imread(os.path.join(data_path, n)) for n in names]
             torch.cuda.synchronize(self.device)
             start_time = time.time()
-            rows = self.detect_bgr_batch(np.stack(frames))
+            if self.input_shape[2] == 1 and all(f.shape == frames[0].shape for f in frames):
+                rows = self.detect_bgr_batch(np.stack(frames))
+            else:
+                rows = self.detect_frames(frames)
             total_time = float(time.time() - start_time) * 1000 / len(names)
             avg_time += total_time * len(names)
             for filename, ori_img, all_bbox_rects in zip(names, frames, rows):
