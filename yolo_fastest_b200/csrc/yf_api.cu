@@ -20,6 +20,7 @@
 #include "yf_tct.cuh"
 #include "yf_wirb.cuh"
 #include "yf_tcpw.cuh"
+#include "yf_tcpw_tma.cuh"
 #include "yf_tcup.cuh"
 #include "yf_tcirb2.cuh"
 #include "yf_tcdense.cuh"
@@ -119,6 +120,7 @@ struct TmaCache {
     const void* ptr = nullptr;
     int B = 0;
     bool u8 = false;
+    int box = 0;                 // box shape the map was encoded for (groups whose tile shape depends on the batch; < 0: encode failed)
     bool failed = false;
 };
 
@@ -528,13 +530,33 @@ cudaError_t init_wstem() {
 template <class C>
 cudaError_t init_wirb() { return cudaFuncSetAttribute(wirb_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES); }
 
+// The depthwise 5x5 -> 1x1 groups take their input by tensor-tile TMA (dwpw_tma_kernel) where the map's rows are a multiple of 16 bytes
+// and the tensor map encodes; otherwise, and in a -DYF_DWPW_TMA=0 build, the cp.async kernel dwpw_tc_kernel. Both read the same packed
+// weights and give the same bits.
+#ifndef YF_DWPW_TMA
+#define YF_DWPW_TMA 1
+#endif
 template <class C>
 void launch_dwpwtc(const GroupArgs& g, const void*, bool, int B, cudaStream_t st) {
     using G = typename C::G;
+    using T = DwPwTmaCfg<C>;
     const int tx = cdiv(g.Wout, G::TW), ty = cdiv(g.Hout, G::TH);
     const int total = B * tx * ty;
     const int grid = total < g.resident ? total : g.resident;
-    launch_k(g.pdl, dwpw_tc_kernel<C>, grid, C::NT, C::SMEM_BYTES, st, g.x, g.y, g.w, g.Hout, g.Wout, tx, ty, total, g.headn > 0 ? g.headn : C::N);
+    const int nout = g.headn > 0 ? g.headn : C::N;
+    bool tma = YF_DWPW_TMA && g.Wout % 4 == 0;
+    if (tma) {
+        TmaCache* tc = g.tc;
+        const int box = T::BW * 1024 + T::BH;
+        if (tc->ptr != g.x || tc->B != B || (tc->box != box && tc->box != -box)) {
+            // an encode failure selects the cp.async kernel for this input (recorded as -box), it is not a forward error
+            const bool ok = tma_make_map4(&tc->map, g.x, 4, B, C::C, g.Hout, g.Wout, T::BW, T::BH, C::MC) == 0;
+            tc->ptr = g.x; tc->B = B; tc->box = ok ? box : -box;
+        }
+        tma = tc->box == box;
+    }
+    if (tma) launch_k(g.pdl, dwpw_tma_kernel<T>, grid, T::NT, T::SMEM_BYTES, st, g.tc->map, g.y, g.w, g.Hout, g.Wout, tx, ty, total, nout);
+    else launch_k(g.pdl, dwpw_tc_kernel<C>, grid, C::NT, C::SMEM_BYTES, st, g.x, g.y, g.w, g.Hout, g.Wout, tx, ty, total, nout);
 }
 template <class CB, class CS, class CN>
 void launch_dwpwtc_auto(const GroupArgs& g, const void* x, bool u8, int B, cudaStream_t st) {      // CS: small batches, CN: narrow maps
@@ -544,9 +566,15 @@ void launch_dwpwtc_auto(const GroupArgs& g, const void* x, bool u8, int B, cudaS
     else if (2 * big <= g.nsm) launch_dwpwtc<CS>(g, x, u8, B, st);
     else launch_dwpwtc<CB>(g, x, u8, B, st);
 }
-template <class C> int occ_dwpwtc() { return occ_of(dwpw_tc_kernel<C>, C::NT, C::SMEM_BYTES); }
+template <class C> int occ_dwpwtc() {
+    return std::min(occ_of(dwpw_tc_kernel<C>, C::NT, C::SMEM_BYTES), occ_of(dwpw_tma_kernel<DwPwTmaCfg<C>>, DwPwTmaCfg<C>::NT, DwPwTmaCfg<C>::SMEM_BYTES));
+}
 template <class C>
-cudaError_t init_dwpwtc() { return cudaFuncSetAttribute(dwpw_tc_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES); }
+cudaError_t init_dwpwtc() {
+    const cudaError_t e = cudaFuncSetAttribute(dwpw_tc_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(dwpw_tma_kernel<DwPwTmaCfg<C>>, cudaFuncAttributeMaxDynamicSharedMemorySize, DwPwTmaCfg<C>::SMEM_BYTES);
+}
 
 template <class C>
 void launch_irbtc2(const GroupArgs& g, const void*, bool, int B, cudaStream_t st) {
