@@ -234,6 +234,37 @@ int yf_detect_host_frames(yf_ctx* ctx, const uint8_t* frames_host, int64_t nbyte
                           const int32_t* Wo, const yf_post_params* p, yf_det* out_host, int32_t* counts_host,
                           int32_t* status_host, void* stream);
 
+/* ---- baseline JPEG files decoded on the device --------------------------------------------------------------------------- */
+
+/* Status bit of yf_decode_jpeg / yf_detect_host_jpeg: the file's entropy-coded data ended early, held an invalid Huffman code, or
+ * missed or misordered an RSTn marker (libjpeg warns and pads with zeros there; the device output of such a file is not cv2's). */
+#define YF_STATUS_JPEG_CORRUPT 4
+
+/* Host only, no CUDA: 0 and the decoded size if the device decoder takes this file, else YF_ERR_ARG with the reason in
+ * yf_last_error(NULL). Taken: baseline sequential Huffman-coded files (SOF0, SOF1) with 8-bit samples and one interleaved scan of
+ * every component; gray, or YCbCr at 4:4:4, 4:2:2 or 4:2:0; restart intervals; files without DHT segments (the T.81 K.3 tables);
+ * sizes 1 .. 16384. Turned down: progressive, arithmetic, lossless and hierarchical files, 12-bit samples, 2 or 4 components,
+ * other sampling factors, several scans, RGB files (Adobe transform 0, or component IDs R, G, B without JFIF / Adobe markers),
+ * EXIF orientations other than 1 (cv2 rotates those), truncated or malformed headers, and bytes that are not a JPEG. */
+int yf_jpeg_probe(const uint8_t* data, int64_t nbytes, int32_t* h, int32_t* w);
+
+/* B JPEG files back to back in HOST memory (file b = bytes [off[b], off[b] + len[b]) of files_host, nbytes in all) ->
+ * the BGR frames cv2.imdecode(IMREAD_COLOR) returns, byte for byte, at frame_off[b] of frames_dev (frames_bytes long; [h, w, 3],
+ * contiguous rows: the layout yf_preprocess_frames reads). status_dev [B]: YF_STATUS_JPEG_CORRUPT. off / len / frame_off are HOST
+ * arrays. Every header is parsed and checked before anything is enqueued; one copy of the nbytes, then 3 kernel launches per 256
+ * files. The decoder reads no byte of a file outside its [off[b], off[b] + len[b]).
+ * Enqueued on `stream`; files_host must stay unchanged until the stream has passed the call. */
+int yf_decode_jpeg(yf_ctx* ctx, const uint8_t* files_host, int64_t nbytes, int B, const int64_t* off, const int64_t* len,
+                   uint8_t* frames_dev, const int64_t* frame_off, int64_t frames_bytes, int32_t* status_dev, void* stream);
+
+/* yf_detect_host_frames for JPEG files: one copy of the files, decode, yf_preprocess_frames, yf_detect, results back in
+ * NETWORK-input coordinates; status_host also carries bit 2 (when status_host is NULL a corrupt file fails the call with
+ * YF_ERR_DOMAIN). frames_host (may be NULL) receives the decoded frames at frame_off, for callers that draw on them.
+ * B <= max_batch. Synchronises `stream`. */
+int yf_detect_host_jpeg(yf_ctx* ctx, const uint8_t* files_host, int64_t nbytes, int B, const int64_t* off, const int64_t* len,
+                        const int64_t* frame_off, const yf_post_params* p, yf_det* out_host, int32_t* counts_host,
+                        int32_t* status_host, uint8_t* frames_host, void* stream);
+
 /* ---- introspection ---------------------------------------------------------------------- */
 
 /* Kernels launched by this ctx since creation (the bench's gpu_launches evidence). */

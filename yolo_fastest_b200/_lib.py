@@ -12,6 +12,7 @@ MODE_DETECT = 0
 MODE_VALIDATE = 1
 VARIANT_FULL = 0
 VARIANT_LITE = 1
+STATUS_JPEG_CORRUPT = 4
 
 
 class YfError(RuntimeError):
@@ -63,6 +64,9 @@ SYMBOLS = [
     ("yf_detect_host_bgr", C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.POINTER(YfPostParams), _P, _P, _P, _P]),
     ("yf_preprocess_frames", C.c_int, [_P, _P, C.c_int, _P, _P, _P, _P, _P]),
     ("yf_detect_host_frames", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.POINTER(YfPostParams), _P, _P, _P, _P]),
+    ("yf_jpeg_probe", C.c_int, [_P, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
+    ("yf_decode_jpeg", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P, C.c_int64, _P, _P]),
+    ("yf_detect_host_jpeg", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.POINTER(YfPostParams), _P, _P, _P, _P, _P]),
     ("yf_compact_dets", C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P]),
     ("yf_launch_count", C.c_int64, [_P]),
     ("yf_profile_forward", C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.c_int]),

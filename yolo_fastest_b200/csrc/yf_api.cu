@@ -26,6 +26,7 @@
 #include "yf_tcdense.cuh"
 #include "yf_tcdense2.cuh"
 #include "yf_prep.cuh"
+#include "yf_jpeg.cuh"
 
 using namespace yf;
 
@@ -215,6 +216,11 @@ struct yf_ctx {
     int prep_Ho = 0, prep_Wo = 0;
     unsigned char* d_bgr = nullptr;
     size_t bgr_cap = 0;
+    int16_t* d_coef = nullptr;                          // JPEG coefficient workspace (128 bytes a block, grow-only, one chunk of files)
+    size_t coef_cap = 0;
+    unsigned char* d_jframes = nullptr;                 // decoded frames of yf_detect_host_jpeg (grow-only)
+    size_t jframes_cap = 0;
+    int32_t* d_jstatus = nullptr;                       // per-file decoder status of yf_detect_host_jpeg [max_batch]
     unsigned char* n_alive = nullptr;                   // yf_nms_sorted_* scratch
     int n_alive_cap = 0;
     int64_t launches = 0;
@@ -1442,6 +1448,8 @@ extern "C" int yf_create_variant(yf_ctx** out, int device, int in_ch, int num_cl
         cudaFuncSetAttribute(post_kernel<POST_SRC_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 12),
         cudaFuncSetAttribute(prep_frames_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
         cudaFuncSetAttribute(prep_frames_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
+        cudaFuncSetAttribute(jpeg_entropy_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, JPEG_TABS_BYTES),
+        cudaFuncSetAttribute(jpeg_entropy_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * JPEG_TABS_BYTES),
         init_irb<CfgRes2>(), init_irb<CfgDown2>(), init_irb<CfgRes3a>(), init_irb<CfgWide3>(),
         init_irb<CfgRes3b>(), init_irbtc<CfgRes3bTc>(), init_irbt<CfgRes3bTt>(), init_irbt<CfgRes4Tt>(), init_irbt<CfgRes3aTt>(), init_irbt<CfgWide3Tt>(), init_irbt<CfgDown3Tt>(), init_irbt<CfgDown4Tt>(), init_irbtc<CfgRes4Tc>(), init_irbtc2<CfgRes5Tc>(), init_irbtc2<CfgRes5TcS>(), init_irbtc2<CfgRes5TcXS>(), init_irbtc2<CfgRes5TcN>(), init_dwpwtc<CfgNeckS1TcS>(), init_dwpwtc<CfgNeckS2TcS>(), init_irbtc<CfgRes3bTcXS>(), init_irbtc<CfgRes4TcXS>(), init_dwpwtc<CfgNeckS1TcN>(), init_dwpwtc<CfgNeckS2TcN>(), init_dwpwtc<CfgNeckL1TcN>(), init_dwpwtc<CfgNeckL2TcN>(), init_irb<CfgDown3N>(), init_irb<CfgDown4N>(), init_dwpwtc<CfgNeckL1TcS>(), init_dwpwtc<CfgNeckL2TcS>(), init_irbtc<CfgRes3bTcS>(), init_irbtc<CfgRes4TcS>(), init_dwpwtc<CfgNeckS1Tc>(), init_dwpwtc<CfgNeckL1Tc>(), init_dwpwtc<CfgNeckS2Tc>(), init_dwpwtc<CfgNeckL2Tc>(), init_irb<CfgDown3>(), init_irb<CfgRes4>(), init_irb<CfgDown4>(), init_irb<CfgRes5>(),
         init_irb<CfgNeckS1>(), init_irb<CfgNeckS2>(), init_irb<CfgNeckL1>(), init_irb<CfgNeckL2>()};
@@ -1461,6 +1469,7 @@ extern "C" void yf_destroy(yf_ctx* ctx) {
     cudaFree(ctx->d_out); cudaFree(ctx->d_counts); cudaFree(ctx->d_status);
     cudaFree(ctx->p_rec); cudaFree(ctx->p_conf); cudaFree(ctx->p_cls); cudaFree(ctx->p_sbox); cudaFree(ctx->p_order);
     cudaFree(ctx->p_alive); cudaFree(ctx->n_alive); cudaFree(ctx->prep_tab); cudaFree(ctx->d_bgr);
+    cudaFree(ctx->d_coef); cudaFree(ctx->d_jframes); cudaFree(ctx->d_jstatus);
     for (auto& kv : ctx->graphs) cudaGraphExecDestroy(kv.second.first);
     if (ctx->s_cap) cudaStreamDestroy(ctx->s_cap);
     if (ctx->s_side) cudaStreamDestroy(ctx->s_side);
@@ -2076,6 +2085,151 @@ extern "C" int yf_detect_host_frames(yf_ctx* ctx, const uint8_t* frames_host, in
     CU(cudaMemcpyAsync(counts_host, ctx->d_counts, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
     if (status_host) CU(cudaMemcpyAsync(status_host, ctx->d_status, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
+    return YF_OK;
+}
+
+// ---- baseline JPEG files decoded on the device (yf_jpeg.cuh): parse every header, one copy of the files, 3 launches per chunk ----------
+extern "C" int yf_jpeg_probe(const uint8_t* data, int64_t nbytes, int32_t* h, int32_t* w) {
+    JpegDesc d;
+    std::string why;
+    if (!jpeg_parse(data, nbytes, d, why)) { set_err(nullptr, "%s", why.c_str()); return YF_ERR_ARG; }
+    if (h) *h = d.h;
+    if (w) *w = d.w;
+    return YF_OK;
+}
+
+// every file's bytes against the buffer, its header through the parser, and (frames_bytes >= 0) its frame against the output buffer
+static int jpeg_check(yf_ctx* ctx, const uint8_t* files, int64_t nbytes, int B, const int64_t* off, const int64_t* len,
+                      const int64_t* frame_off, int64_t frames_bytes, std::vector<JpegDesc>& ds) {
+    if (!files || !off || !len || !frame_off) { set_err(&ctx->err, "null file or descriptor array"); return YF_ERR_ARG; }
+    if (B < 1) { set_err(&ctx->err, "batch %d < 1", B); return YF_ERR_ARG; }
+    ds.resize(B);
+    std::string why;
+    for (int b = 0; b < B; ++b) {
+        if (off[b] < 0 || len[b] < 1 || off[b] > nbytes - len[b]) {
+            set_err(&ctx->err, "file %d: bytes [%lld, %lld) outside the %lld-byte buffer", b, (long long)off[b], (long long)(off[b] + len[b]),
+                    (long long)nbytes);
+            return YF_ERR_ARG;
+        }
+        if (!jpeg_parse(files + off[b], len[b], ds[b], why)) { set_err(&ctx->err, "file %d: %s", b, why.c_str()); return YF_ERR_ARG; }
+        const int64_t size = (int64_t)ds[b].h * ds[b].w * 3;
+        if (frame_off[b] < 0 || (frames_bytes >= 0 && frame_off[b] > frames_bytes - size)) {
+            set_err(&ctx->err, "frame %d: bytes [%lld, %lld) outside the %lld-byte frame buffer", b, (long long)frame_off[b],
+                    (long long)(frame_off[b] + size), (long long)frames_bytes);
+            return YF_ERR_ARG;
+        }
+        ds[b].src = off[b];
+        ds[b].dst = frame_off[b];
+    }
+    return YF_OK;
+}
+
+// Files per warp of the entropy kernel: 1 (the default, DESIGN.md §5.7) or 32; YF_JPEG_FILES_PER_WARP selects the other for timing.
+static int jpeg_fpw() {
+    const char* e = getenv("YF_JPEG_FILES_PER_WARP");
+    return e && atoi(e) == 32 ? 32 : 1;
+}
+
+// files dev (staged) -> frames dev, status dev [B]. The coefficient workspace holds one chunk and is reused in stream order.
+static int jpeg_enqueue(yf_ctx* ctx, const uint8_t* files, std::vector<JpegDesc>& ds, uint8_t* frames, int32_t* status, cudaStream_t st) {
+    const int B = (int)ds.size();
+    int64_t most = 0;
+    for (int c0 = 0; c0 < B; c0 += JPEG_CHUNK) {
+        int64_t blocks = 0;
+        for (int i = c0; i < std::min(B, c0 + JPEG_CHUNK); ++i) { ds[i].cbase = blocks; blocks += jpeg_blocks(ds[i]); }
+        most = std::max(most, blocks);
+    }
+    const size_t need = (size_t)most * 128;
+    if (need > ctx->coef_cap) {
+        CU(cudaStreamSynchronize(st));                  // an earlier call's kernels may still use the old workspace
+        if (ctx->d_coef) CU(cudaFree(ctx->d_coef));
+        ctx->d_coef = nullptr; ctx->coef_cap = 0;
+        CU(cudaMalloc(&ctx->d_coef, need));
+        ctx->coef_cap = need;
+    }
+    const int fpw = jpeg_fpw();
+    JpegChunk ch;
+    for (int c0 = 0; c0 < B; c0 += JPEG_CHUNK) {
+        const int n = std::min(JPEG_CHUNK, B - c0);
+        int64_t max_blocks = 1, max_px = 1;
+        for (int i = 0; i < n; ++i) {
+            ch.d[i] = ds[c0 + i];
+            max_blocks = std::max(max_blocks, jpeg_blocks(ch.d[i]));
+            max_px = std::max(max_px, (int64_t)ch.d[i].h * ch.d[i].w);
+        }
+        if (fpw == 32) jpeg_entropy_kernel<32><<<(n + 31) / 32, 32, 32 * JPEG_TABS_BYTES, st>>>(files, ch, n, ctx->d_coef, status + c0);
+        else jpeg_entropy_kernel<1><<<n, 32, JPEG_TABS_BYTES, st>>>(files, ch, n, ctx->d_coef, status + c0);
+        CU(cudaGetLastError());
+        const dim3 gi((unsigned)std::min<int64_t>((max_blocks + JPEG_IDCT_NT - 1) / JPEG_IDCT_NT, 2048), (unsigned)n);
+        jpeg_idct_kernel<<<gi, JPEG_IDCT_NT, 0, st>>>(files, ch, ctx->d_coef);
+        CU(cudaGetLastError());
+        const dim3 gc((unsigned)std::min<int64_t>((max_px + JPEG_COLOR_NT - 1) / JPEG_COLOR_NT, 4096), (unsigned)n);
+        jpeg_color_kernel<<<gc, JPEG_COLOR_NT, 0, st>>>(ch, ctx->d_coef, frames);
+        CU(cudaGetLastError());
+        ctx->launches += 3;
+    }
+    return YF_OK;
+}
+
+extern "C" int yf_decode_jpeg(yf_ctx* ctx, const uint8_t* files_host, int64_t nbytes, int B, const int64_t* off, const int64_t* len,
+                              uint8_t* frames_dev, const int64_t* frame_off, int64_t frames_bytes, int32_t* status_dev, void* stream) {
+    CTX_CHECK(ctx);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!frames_dev || !status_dev) { set_err(&ctx->err, "null frames or status pointer"); return YF_ERR_ARG; }
+    std::vector<JpegDesc> ds;
+    int rc = jpeg_check(ctx, files_host, nbytes, B, off, len, frame_off, frames_bytes, ds);
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    if ((rc = ensure_bgr(ctx, (size_t)nbytes, st))) return rc;
+    CU(cudaMemcpyAsync(ctx->d_bgr, files_host, (size_t)nbytes, cudaMemcpyHostToDevice, st));       // the files, one copy
+    return jpeg_enqueue(ctx, ctx->d_bgr, ds, frames_dev, status_dev, st);
+}
+
+extern "C" int yf_detect_host_jpeg(yf_ctx* ctx, const uint8_t* files_host, int64_t nbytes, int B, const int64_t* off, const int64_t* len,
+                                   const int64_t* frame_off, const yf_post_params* p, yf_det* out_host, int32_t* counts_host,
+                                   int32_t* status_host, uint8_t* frames_host, void* stream) {
+    CTX_CHECK(ctx);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!p || !out_host || !counts_host) { set_err(&ctx->err, "null argument"); return YF_ERR_ARG; }
+    if (p->max_det < 1) { set_err(&ctx->err, "max_det must be >= 1"); return YF_ERR_ARG; }
+    if (B < 1 || B > ctx->max_batch) { set_err(&ctx->err, "batch %d outside [1, max_batch=%d]", B, ctx->max_batch); return YF_ERR_ARG; }
+    std::vector<JpegDesc> ds;
+    int rc = jpeg_check(ctx, files_host, nbytes, B, off, len, frame_off, -1, ds);
+    if (rc) return rc;
+    std::vector<int32_t> Ho(B), Wo(B);
+    int64_t frames_bytes = 0;
+    for (int b = 0; b < B; ++b) {
+        Ho[b] = ds[b].h; Wo[b] = ds[b].w;
+        frames_bytes = std::max(frames_bytes, frame_off[b] + (int64_t)Ho[b] * Wo[b] * 3);
+    }
+    CU(cudaSetDevice(ctx->device));
+    if (!ctx->weights_loaded) { set_err(&ctx->err, "yf_load_weights has not been called"); return YF_ERR_STATE; }
+    ORDER(ctx, st);
+    if ((rc = ensure_out(ctx, p->max_det))) return rc;
+    if ((rc = ensure_bgr(ctx, (size_t)nbytes, st))) return rc;
+    if ((size_t)frames_bytes > ctx->jframes_cap) {
+        CU(cudaStreamSynchronize(st));                  // an earlier call's kernels may still read the old frames
+        if (ctx->d_jframes) CU(cudaFree(ctx->d_jframes));
+        ctx->d_jframes = nullptr; ctx->jframes_cap = 0;
+        CU(cudaMalloc(&ctx->d_jframes, (size_t)frames_bytes));
+        ctx->jframes_cap = (size_t)frames_bytes;
+    }
+    if (!ctx->d_jstatus) CU(cudaMalloc(&ctx->d_jstatus, sizeof(int32_t) * ctx->max_batch));
+    CU(cudaMemcpyAsync(ctx->d_bgr, files_host, (size_t)nbytes, cudaMemcpyHostToDevice, st));       // the files, one copy
+    if ((rc = jpeg_enqueue(ctx, ctx->d_bgr, ds, ctx->d_jframes, ctx->d_jstatus, st))) return rc;
+    if ((rc = frames_enqueue(ctx, ctx->d_jframes, B, frame_off, Ho.data(), Wo.data(), ctx->d_u8, st))) return rc;
+    if ((rc = detect_fixed(ctx, ctx->d_u8, true, B, p, ctx->d_out, ctx->d_counts, ctx->d_status, st))) return rc;
+    std::vector<int32_t> jst(B);
+    CU(cudaMemcpyAsync(out_host, ctx->d_out, sizeof(yf_det) * (size_t)B * p->max_det, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(counts_host, ctx->d_counts, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    if (status_host) CU(cudaMemcpyAsync(status_host, ctx->d_status, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(jst.data(), ctx->d_jstatus, sizeof(int32_t) * B, cudaMemcpyDeviceToHost, st));
+    if (frames_host) CU(cudaMemcpyAsync(frames_host, ctx->d_jframes, (size_t)frames_bytes, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    for (int b = 0; b < B; ++b) {
+        if (status_host) status_host[b] |= jst[b];
+        else if (jst[b]) { set_err(&ctx->err, "file %d: corrupt entropy-coded data", b); return YF_ERR_DOMAIN; }
+    }
     return YF_OK;
 }
 

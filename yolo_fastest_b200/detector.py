@@ -209,6 +209,49 @@ def frame_layout(frames):
     return off, Ho, Wo, int(off[-1]) + int(Ho[-1]) * int(Wo[-1]) * 3
 
 
+def jpeg_probe(data):
+    """-> (h, w) if the device JPEG decoder takes this file (bytes / uint8 buffer), else YfError with the header parser's reason
+    (progressive, arithmetic, 12-bit, CMYK, 4:1:1, several scans, RGB, EXIF-rotated, truncated, not a JPEG ...). Host only."""
+    buf = np.frombuffer(data, np.uint8) if isinstance(data, (bytes, bytearray, memoryview)) else np.ascontiguousarray(data, np.uint8).reshape(-1)
+    h, w = C.c_int32(), C.c_int32()
+    if _lib.lib().yf_jpeg_probe(buf.ctypes.data if buf.size else None, buf.size, C.byref(h), C.byref(w)) != 0:
+        raise _lib.YfError(_lib.lib().yf_last_error(None).decode())
+    return h.value, w.value
+
+
+def _file_bytes(f):
+    """a path, bytes or a uint8 numpy buffer -> bytes"""
+    if isinstance(f, (str, os.PathLike)):
+        with open(f, "rb") as fh:
+            return fh.read()
+    if isinstance(f, (bytes, bytearray, memoryview)):
+        return bytes(f)
+    if isinstance(f, np.ndarray) and f.dtype == np.uint8:
+        return f.tobytes()
+    raise _lib.YfError("a JPEG file is a path, bytes or a uint8 numpy buffer, not %s" % type(f).__name__)
+
+
+def jpeg_layout(datas):
+    """Probe every file and lay the files and their decoded frames out back to back -> (files uint8 [nbytes], off int64 [B],
+    len int64 [B], frame_off int64 [B], Ho int32 [B], Wo int32 [B], frames_bytes). Raises YfError naming the first file not taken."""
+    if not datas:
+        raise _lib.YfError("files: a non-empty list")
+    B = len(datas)
+    off, ln, foff = np.zeros(B, np.int64), np.zeros(B, np.int64), np.zeros(B, np.int64)
+    Ho, Wo = np.zeros(B, np.int32), np.zeros(B, np.int32)
+    pos = fpos = 0
+    for b, d in enumerate(datas):
+        try:
+            Ho[b], Wo[b] = jpeg_probe(d)
+        except _lib.YfError as e:
+            raise _lib.YfError("file %d: %s" % (b, e)) from None
+        off[b], ln[b], foff[b] = pos, len(d), fpos
+        pos += len(d)
+        fpos += -(-int(Ho[b]) * int(Wo[b]) * 3 // FRAME_ALIGN) * FRAME_ALIGN
+    files = np.frombuffer(b"".join(datas), np.uint8)
+    return files, off, ln, foff, Ho, Wo, int(foff[-1]) + int(Ho[-1]) * int(Wo[-1]) * 3
+
+
 def pack_frames(frames, dst, off):
     """Copy host frames into the uint8 numpy buffer `dst` at the offsets of frame_layout (any strides)."""
     for f, o in zip(frames, off):
@@ -408,6 +451,75 @@ class Detect_YOLO:
                     r[3] = round(r[3] * scale_h)
         return rows
 
+    # ---- JPEG files decoded on the device (yf_decode_jpeg / yf_detect_host_jpeg) ---------------------------------------------------
+    def decode_jpeg(self, files):
+        """JPEG files (paths, bytes or uint8 numpy buffers) -> list of cuda uint8 [h, w, 3] BGR tensors, byte-identical to
+        cv2.imread / cv2.imdecode(IMREAD_COLOR). Every header is checked first (jpeg_probe); a file the decoder does not take raises
+        YfError naming its index before anything runs on the device, and a file whose scan data is corrupt raises after the decode."""
+        datas = [_file_bytes(f) for f in files]
+        files_u8, off, ln, foff, Ho, Wo, fbytes = jpeg_layout(datas)
+        B = len(datas)
+        H, W = self.input_shape[0:2]
+        ctx = self.model.context(self.device, H, W, B)
+        frames = torch.empty((fbytes,), dtype=torch.uint8, device=self.device)
+        status = torch.zeros((B,), dtype=torch.int32, device=self.device)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().yf_decode_jpeg(ctx.handle, files_u8.ctypes.data, files_u8.size, B, off.ctypes.data, ln.ctypes.data,
+                                                frames.data_ptr(), foff.ctypes.data, fbytes, status.data_ptr(), C.c_void_p(stream)),
+                       ctx.handle)
+        st = status.cpu().numpy()         # synchronises the stream, so files_u8 may go
+        bad = np.nonzero(st & _lib.STATUS_JPEG_CORRUPT)[0]
+        if bad.size:
+            raise _lib.YfError("file %d: corrupt JPEG entropy-coded data" % int(bad[0]))
+        return [frames[int(o):int(o) + int(h) * int(w) * 3].view(int(h), int(w), 3) for o, h, w in zip(foff, Ho, Wo)]
+
+    def detect_jpeg(self, files, max_det=64, raw=False, adjust=True, return_frames=False):
+        """JPEG files (paths, bytes or uint8 numpy buffers) -> per-image rows equal to detect_frames([cv2.imread(f) ...]): one
+        yf_detect_host_jpeg call (one copy of the files, decode, pre-processing, forward, decode, NMS, the result slab back), for gray
+        and colour networks. adjust as in detect_frames. With return_frames=True also returns the decoded BGR frames (host numpy), for
+        drawing. A file the decoder does not take raises YfError naming its index; nothing is launched then."""
+        datas = [_file_bytes(f) for f in files]
+        files_u8, off, ln, foff, Ho, Wo, fbytes = jpeg_layout(datas)
+        rows, frames = self._detect_jpeg(files_u8, off, ln, foff, Ho, Wo, fbytes, max_det, return_frames)
+        if not raw:
+            rows = [_rows_from_dets(d) for d in rows]
+            if adjust:
+                H, W = self.input_shape[0:2]
+                for rr, h, w in zip(rows, Ho, Wo):
+                    if [int(h), int(w)] == [H, W]:
+                        continue
+                    scale_h, scale_w = int(h) / H, int(w) / W
+                    for r in rr:
+                        r[0] = round(r[0] * scale_w)
+                        r[2] = round(r[2] * scale_w)
+                        r[1] = round(r[1] * scale_h)
+                        r[3] = round(r[3] * scale_h)
+        return (rows, frames) if return_frames else rows
+
+    def _detect_jpeg(self, files_u8, off, ln, foff, Ho, Wo, fbytes, max_det, want_frames):
+        B = len(off)
+        H, W = self.input_shape[0:2]
+        ctx = self.model.context(self.device, H, W, B)
+        pin_out = torch.empty((B, max_det, _lib.DET_DTYPE.itemsize), dtype=torch.uint8).pin_memory()
+        pin_cnt = torch.empty((B,), dtype=torch.int32).pin_memory()
+        pin_st = torch.empty((B,), dtype=torch.int32).pin_memory()
+        frames = np.empty((fbytes,), np.uint8) if want_frames else None
+        p = self.post_process._params(_lib.MODE_DETECT, max_det)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().yf_detect_host_jpeg(ctx.handle, files_u8.ctypes.data, files_u8.size, B, off.ctypes.data, ln.ctypes.data,
+                                                     foff.ctypes.data, C.byref(p), pin_out.data_ptr(), pin_cnt.data_ptr(), pin_st.data_ptr(),
+                                                     frames.ctypes.data if want_frames else None, C.c_void_p(stream)), ctx.handle)
+        bad = np.nonzero(pin_st.numpy() & _lib.STATUS_JPEG_CORRUPT)[0]
+        if bad.size:
+            raise _lib.YfError("file %d: corrupt JPEG entropy-coded data" % int(bad[0]))
+        res = _finish(pin_out, pin_cnt, pin_st, B, max_det,
+                      lambda need: self._detect_jpeg(files_u8, off, ln, foff, Ho, Wo, fbytes, need, False)[0])
+        if want_frames:
+            frames = [frames[int(o):int(o) + int(h) * int(w) * 3].reshape(int(h), int(w), 3) for o, h, w in zip(foff, Ho, Wo)]
+        return res, frames
+
     # ---- batched detection through the C ABI with host buffers -----------------------------------------
     def detect_batch(self, u8_batch, max_det=64, raw=False):
         """uint8 images [B, H, W] (gray) or [B, 3, H, W] (RGB planes, 3-channel networks), host numpy array or host torch
@@ -562,22 +674,42 @@ class Detect_YOLO:
 
             self.logger.info("detect avg_time: %.2fms" % (avg_time / num))
 
+    # Smallest batch the file driver decodes on the device. One thread decodes a whole file, so a batch costs at least one file's
+    # decode (12 ms for a shipped 640x512 file, DESIGN.md §5.7): on 1024 files the device path took 1.80 s against 2.42 s for
+    # cv2.imread at batch 32, and 2.87 s against 2.05 s at batch 8 (profiles/r04_jpeg.txt).
+    JPEG_MIN_BATCH = 32
+
     def batch_detect_batched(self, data_path, result_path, batch_size=32):
-        """batch_detect with the per-file loop turned into batches (SURVEY 8f-1): the frames of `batch_size` files are
-        decoded on the host (cv2.imread), everything else - gray, resize, normalisation, forward, decode, NMS - is ONE
-        yf_detect_host_bgr call per batch. Same result files and log lines as batch_detect (detect.py:141-192); the two
-        per-image times of the log line are the batch's time divided by its size. A batch whose frames differ in size, or any batch
-        of a 3-channel network, goes through detect_frames instead (boxes scaled to each frame's own size)."""
+        """batch_detect with the per-file loop turned into batches (SURVEY 8f-1). When a batch holds at least JPEG_MIN_BATCH files and
+        the device decoder takes every one of them (jpeg_probe), the batch is ONE yf_detect_host_jpeg call: JPEG decode, gray / resize, normalisation, forward, decode and NMS on
+        the device, the decoded frames back for drawing. Any other batch (PNGs, progressive or EXIF-rotated JPEGs, ...) is decoded on
+        the host (cv2.imread) and is one yf_detect_host_bgr call, or one detect_frames call when its frames differ in size or the
+        network is 3-channel (boxes scaled to each frame's own size). Same result files and log lines as batch_detect
+        (detect.py:141-192); the two per-image times of the log line are the batch's time divided by its size, and include the
+        decode on the device path."""
         import cv2
         img_list = os.listdir(data_path)
         num = len(img_list)
         avg_time = 0
         for i0 in range(0, num, batch_size):
             names = img_list[i0:i0 + batch_size]
-            frames = [cv2.imread(os.path.join(data_path, n)) for n in names]
+            datas = []
+            for n in names:
+                with open(os.path.join(data_path, n), "rb") as f:
+                    datas.append(f.read())
+            on_device = len(names) >= self.JPEG_MIN_BATCH
+            if on_device:
+                try:
+                    jpeg_layout(datas)
+                except _lib.YfError:
+                    on_device = False
+            if not on_device:
+                frames = [cv2.imread(os.path.join(data_path, n)) for n in names]
             torch.cuda.synchronize(self.device)
             start_time = time.time()
-            if self.input_shape[2] == 1 and all(f.shape == frames[0].shape for f in frames):
+            if on_device:
+                rows, frames = self.detect_jpeg(datas, return_frames=True)
+            elif self.input_shape[2] == 1 and all(f.shape == frames[0].shape for f in frames):
                 rows = self.detect_bgr_batch(np.stack(frames))
             else:
                 rows = self.detect_frames(frames)
