@@ -265,6 +265,38 @@ int yf_detect_host_jpeg(yf_ctx* ctx, const uint8_t* files_host, int64_t nbytes, 
                         const int64_t* frame_off, const yf_post_params* p, yf_det* out_host, int32_t* counts_host,
                         int32_t* status_host, uint8_t* frames_host, void* stream);
 
+/* ---- baseline JPEG files encoded on the device -------------------------------------------------------------------------- */
+
+/* Chroma sampling of the encoder, with the values of cv2.IMWRITE_JPEG_SAMPLING_FACTOR_* so that callers can pass those through. */
+#define YF_JPEG_SAMPLING_420 0x221111   /* = cv2.IMWRITE_JPEG_SAMPLING_FACTOR_420, cv2's default */
+#define YF_JPEG_SAMPLING_422 0x211111
+#define YF_JPEG_SAMPLING_444 0x111111
+
+/* Host only, no CUDA: the most bytes one encoded file of an h x w frame can take (headers, every scan byte stuffed, EOI), or
+ * YF_ERR_ARG (size outside [1, 16384], other sampling factors) with the reason in yf_last_error(NULL). */
+int64_t yf_jpeg_encode_bound(int h, int w, int sampling);
+/* Host only: the header bytes (SOI .. SOS) cv2.imencode writes for these parameters into out (cap bytes); returns their length (623)
+ * or YF_ERR_ARG (quality outside [1, 100], other sampling factors, size outside [1, 16384], cap too small). */
+int yf_jpeg_encode_header(int h, int w, int quality, int sampling, uint8_t* out, int64_t cap);
+/* B BGR uint8 frames in DEVICE memory (frame b at byte offset frame_off[b] of frames_dev, [h[b], w[b], 3], contiguous rows: the layout
+ * yf_decode_jpeg writes and yf_preprocess_frames reads) -> B JPEG files, each byte for byte what
+ * cv2.imencode(".jpg", frame, [IMWRITE_JPEG_QUALITY, quality, IMWRITE_JPEG_SAMPLING_FACTOR, sampling]) returns: baseline, standard
+ * Huffman tables, no restart intervals, JFIF APP0. File b goes to out_dev + out_off[b], which must have room for
+ * yf_jpeg_encode_bound bytes inside the out_bytes of out_dev; len_dev [B] int64 (device) receives the length of each file.
+ * frame_off / h / w / out_off are HOST arrays; every argument is checked before anything is enqueued. 4 kernel launches per 256
+ * frames. Enqueued on `stream`. The frames are BGR [h, w, 3] by construction, and the entry points have no parameter for restart
+ * intervals, optimised or progressive coding or a separate chroma quality: those outputs are not produced. */
+int yf_encode_jpeg(yf_ctx* ctx, const uint8_t* frames_dev, int B, const int64_t* frame_off, const int32_t* h, const int32_t* w,
+                   int quality, int sampling, uint8_t* out_dev, const int64_t* out_off, int64_t out_bytes, int64_t* len_dev,
+                   void* stream);
+/* The same from HOST frames (frames_host, nbytes long; every frame must lie inside): one copy of the nbytes to the device, the encode,
+ * the lengths back into len_host [B], then ONE copy of the files packed back to back (file b right after file b - 1) into out_host.
+ * When the files take more than `cap` bytes the call fails with YF_ERR_ARG naming the need, len_host holds the lengths, and nothing is
+ * written to out_host. Synchronises `stream`. */
+int yf_encode_host_jpeg(yf_ctx* ctx, const uint8_t* frames_host, int64_t nbytes, int B, const int64_t* frame_off,
+                        const int32_t* h, const int32_t* w, int quality, int sampling, uint8_t* out_host, int64_t cap,
+                        int64_t* len_host, void* stream);
+
 /* ---- introspection ---------------------------------------------------------------------- */
 
 /* Kernels launched by this ctx since creation (the bench's gpu_launches evidence). */

@@ -13,6 +13,9 @@ MODE_VALIDATE = 1
 VARIANT_FULL = 0
 VARIANT_LITE = 1
 STATUS_JPEG_CORRUPT = 4
+JPEG_SAMPLING_420 = 0x221111      # = cv2.IMWRITE_JPEG_SAMPLING_FACTOR_420 (and _422, _444 below): yf_encode_jpeg takes cv2's values
+JPEG_SAMPLING_422 = 0x211111
+JPEG_SAMPLING_444 = 0x111111
 
 
 class YfError(RuntimeError):
@@ -67,6 +70,10 @@ SYMBOLS = [
     ("yf_jpeg_probe", C.c_int, [_P, C.c_int64, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     ("yf_decode_jpeg", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, _P, C.c_int64, _P, _P]),
     ("yf_detect_host_jpeg", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.POINTER(YfPostParams), _P, _P, _P, _P, _P]),
+    ("yf_jpeg_encode_bound", C.c_int64, [C.c_int, C.c_int, C.c_int]),
+    ("yf_jpeg_encode_header", C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int64]),
+    ("yf_encode_jpeg", C.c_int, [_P, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P, C.c_int64, _P, _P]),
+    ("yf_encode_host_jpeg", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, C.c_int64, _P, _P]),
     ("yf_compact_dets", C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P]),
     ("yf_launch_count", C.c_int64, [_P]),
     ("yf_profile_forward", C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.c_int]),

@@ -27,6 +27,7 @@
 #include "yf_tcdense2.cuh"
 #include "yf_prep.cuh"
 #include "yf_jpeg.cuh"
+#include "yf_jpeg_enc.cuh"
 
 using namespace yf;
 
@@ -221,6 +222,18 @@ struct yf_ctx {
     unsigned char* d_jframes = nullptr;                 // decoded frames of yf_detect_host_jpeg (grow-only)
     size_t jframes_cap = 0;
     int32_t* d_jstatus = nullptr;                       // per-file decoder status of yf_detect_host_jpeg [max_batch]
+    // JPEG encoding (yf_jpeg_enc.cuh), all grow-only: coefficients, bit offsets and bit buffers of one chunk of frames; the header
+    // bytes of a call; the files and lengths of yf_encode_host_jpeg before and after packing
+    unsigned char* d_jenc = nullptr;
+    size_t jenc_cap = 0;
+    unsigned char* d_jhdr = nullptr;
+    size_t jhdr_cap = 0;
+    unsigned char* d_jout = nullptr;
+    size_t jout_cap = 0;
+    unsigned char* d_jpack = nullptr;
+    size_t jpack_cap = 0;
+    int64_t* d_jlen = nullptr;
+    size_t jlen_cap = 0;
     unsigned char* n_alive = nullptr;                   // yf_nms_sorted_* scratch
     int n_alive_cap = 0;
     int64_t launches = 0;
@@ -1470,6 +1483,7 @@ extern "C" void yf_destroy(yf_ctx* ctx) {
     cudaFree(ctx->p_rec); cudaFree(ctx->p_conf); cudaFree(ctx->p_cls); cudaFree(ctx->p_sbox); cudaFree(ctx->p_order);
     cudaFree(ctx->p_alive); cudaFree(ctx->n_alive); cudaFree(ctx->prep_tab); cudaFree(ctx->d_bgr);
     cudaFree(ctx->d_coef); cudaFree(ctx->d_jframes); cudaFree(ctx->d_jstatus);
+    cudaFree(ctx->d_jenc); cudaFree(ctx->d_jhdr); cudaFree(ctx->d_jout); cudaFree(ctx->d_jpack); cudaFree(ctx->d_jlen);
     for (auto& kv : ctx->graphs) cudaGraphExecDestroy(kv.second.first);
     if (ctx->s_cap) cudaStreamDestroy(ctx->s_cap);
     if (ctx->s_side) cudaStreamDestroy(ctx->s_side);
@@ -2230,6 +2244,196 @@ extern "C" int yf_detect_host_jpeg(yf_ctx* ctx, const uint8_t* files_host, int64
         if (status_host) status_host[b] |= jst[b];
         else if (jst[b]) { set_err(&ctx->err, "file %d: corrupt entropy-coded data", b); return YF_ERR_DOMAIN; }
     }
+    return YF_OK;
+}
+
+// ---- JPEG files encoded on the device (yf_jpeg_enc.cuh): headers built on the host, 4 launches per chunk of 256 frames ------------
+static int jpeg_enc_params(std::string* err, int quality, int sampling, int& hs, int& vs) {
+    if (quality < 1 || quality > 100) { set_err(err, "quality %d outside [1, 100]", quality); return YF_ERR_ARG; }
+    if (!jpeg_enc_sampling(sampling, hs, vs)) {
+        set_err(err, "sampling factor 0x%x is not supported (0x221111 4:2:0, 0x211111 4:2:2 and 0x111111 4:4:4 are)", sampling);
+        return YF_ERR_ARG;
+    }
+    return YF_OK;
+}
+
+static bool jpeg_enc_size_ok(int h, int w) { return h >= 1 && w >= 1 && h <= JPEG_MAX_SIDE && w <= JPEG_MAX_SIDE; }
+
+extern "C" int64_t yf_jpeg_encode_bound(int h, int w, int sampling) {
+    int hs, vs;
+    if (jpeg_enc_params(nullptr, 95, sampling, hs, vs)) return YF_ERR_ARG;
+    if (!jpeg_enc_size_ok(h, w)) { set_err(nullptr, "size %dx%d outside [1, %d]", h, w, JPEG_MAX_SIDE); return YF_ERR_ARG; }
+    return jpeg_enc_file_max(h, w, hs, vs);
+}
+
+extern "C" int yf_jpeg_encode_header(int h, int w, int quality, int sampling, uint8_t* out, int64_t cap) {
+    int hs, vs;
+    if (jpeg_enc_params(nullptr, quality, sampling, hs, vs)) return YF_ERR_ARG;
+    if (!jpeg_enc_size_ok(h, w)) { set_err(nullptr, "size %dx%d outside [1, %d]", h, w, JPEG_MAX_SIDE); return YF_ERR_ARG; }
+    if (!out || cap < JPEG_ENC_HEADER_BYTES) { set_err(nullptr, "the header takes %d bytes, cap is %lld", JPEG_ENC_HEADER_BYTES, (long long)cap); return YF_ERR_ARG; }
+    return jpeg_enc_header(h, w, quality, hs, vs, out);
+}
+
+// every frame's size, its bytes against the frames buffer (frames_bytes >= 0) and, with out_off, its file against the output buffer
+static int jpeg_enc_check(yf_ctx* ctx, int B, const int64_t* frame_off, const int32_t* h, const int32_t* w, int64_t frames_bytes, int hs,
+                          int vs, const int64_t* out_off, int64_t out_bytes) {
+    if (!frame_off || !h || !w) { set_err(&ctx->err, "null descriptor array"); return YF_ERR_ARG; }
+    if (B < 1) { set_err(&ctx->err, "batch %d < 1", B); return YF_ERR_ARG; }
+    for (int b = 0; b < B; ++b) {
+        if (!jpeg_enc_size_ok(h[b], w[b])) { set_err(&ctx->err, "frame %d: size %dx%d outside [1, %d]", b, h[b], w[b], JPEG_MAX_SIDE); return YF_ERR_ARG; }
+        const int64_t size = (int64_t)h[b] * w[b] * 3;
+        if (frame_off[b] < 0 || (frames_bytes >= 0 && frame_off[b] > frames_bytes - size)) {
+            set_err(&ctx->err, "frame %d: bytes [%lld, %lld) outside the %lld-byte buffer", b, (long long)frame_off[b],
+                    (long long)(frame_off[b] + size), (long long)frames_bytes);
+            return YF_ERR_ARG;
+        }
+        const int64_t bound = jpeg_enc_file_max(h[b], w[b], hs, vs);
+        if (out_off && (out_off[b] < 0 || out_off[b] > out_bytes - bound)) {
+            set_err(&ctx->err, "frame %d: file bytes [%lld, %lld) (yf_jpeg_encode_bound) outside the %lld-byte output buffer", b,
+                    (long long)out_off[b], (long long)(out_off[b] + bound), (long long)out_bytes);
+            return YF_ERR_ARG;
+        }
+    }
+    return YF_OK;
+}
+
+static int jpeg_enc_grow(yf_ctx* ctx, unsigned char** p, size_t* cap, size_t need) {
+    if (need <= *cap) return YF_OK;
+    CU(cudaDeviceSynchronize());                        // an earlier call's kernels, on any stream, may still use the old buffer
+    if (*p) CU(cudaFree(*p));
+    *p = nullptr; *cap = 0;
+    CU(cudaMalloc(p, need));
+    *cap = need;
+    return YF_OK;
+}
+
+// frames dev -> files at out + out_off[b], len dev [B]. Arguments already checked.
+static int jpeg_enc_enqueue(yf_ctx* ctx, const uint8_t* frames, int B, const int64_t* frame_off, const int32_t* h, const int32_t* w,
+                            int quality, int hs, int vs, uint8_t* out, const int64_t* out_off, int64_t* len, cudaStream_t st) {
+    std::map<std::pair<int, int>, int32_t> hofs;        // one header per distinct size, all staged with one copy
+    std::vector<uint8_t> hb;
+    std::vector<JpegEncDesc> ds(B);
+    for (int b = 0; b < B; ++b) {
+        auto it = hofs.find({h[b], w[b]});
+        if (it == hofs.end()) {
+            it = hofs.emplace(std::make_pair(h[b], w[b]), (int32_t)hb.size()).first;
+            hb.resize(hb.size() + JPEG_ENC_HEADER_BYTES);
+            jpeg_enc_header(h[b], w[b], quality, hs, vs, hb.data() + it->second);
+        }
+        JpegEncDesc& d = ds[b];
+        memset(&d, 0, sizeof d);
+        d.src = frame_off[b]; d.dst = out_off[b];
+        d.hdr = it->second; d.hdr_len = JPEG_ENC_HEADER_BYTES;
+        d.h = (uint16_t)h[b]; d.w = (uint16_t)w[b]; d.hs = (uint8_t)hs; d.vs = (uint8_t)vs;
+        d.mcux = (uint16_t)((w[b] + 8 * hs - 1) / (8 * hs)); d.mcuy = (uint16_t)((h[b] + 8 * vs - 1) / (8 * vs));
+    }
+    // workspace of the largest chunk: [coefficients, 128 B a block | bit offsets, 8 B a block | bit counts of the frames | bit buffers]
+    int64_t most_blocks = 0, most_bits = 0;
+    for (int c0 = 0; c0 < B; c0 += JPEG_ENC_CHUNK) {
+        int64_t blocks = 0, bytes = 0;
+        for (int i = c0; i < std::min(B, c0 + JPEG_ENC_CHUNK); ++i) {
+            ds[i].cbase = blocks; ds[i].bbase = bytes;
+            blocks += jpeg_enc_blocks(h[i], w[i], hs, vs);
+            bytes += (jpeg_enc_scan_max(h[i], w[i], hs, vs) + 31) / 16 * 16;      // whole 16-byte loads of the stuffing stage
+        }
+        most_blocks = std::max(most_blocks, blocks);
+        most_bits = std::max(most_bits, bytes);
+    }
+    // every part starts on a 256-byte boundary: the stuffing kernel reads the bit buffers with 16-byte loads
+    auto up = [](size_t x) { return (x + 255) / 256 * 256; };
+    const size_t off_offs = up((size_t)most_blocks * 128), off_fbits = up(off_offs + (size_t)most_blocks * 8);
+    const size_t off_bits = up(off_fbits + sizeof(int64_t) * JPEG_ENC_CHUNK);
+    int rc = jpeg_enc_grow(ctx, &ctx->d_jenc, &ctx->jenc_cap, off_bits + (size_t)most_bits);
+    if (rc) return rc;
+    if ((rc = jpeg_enc_grow(ctx, &ctx->d_jhdr, &ctx->jhdr_cap, hb.size()))) return rc;
+    CU(cudaMemcpyAsync(ctx->d_jhdr, hb.data(), hb.size(), cudaMemcpyHostToDevice, st));
+    int16_t* coef = reinterpret_cast<int16_t*>(ctx->d_jenc);
+    int64_t* offs = reinterpret_cast<int64_t*>(ctx->d_jenc + off_offs);
+    int64_t* fbits = reinterpret_cast<int64_t*>(ctx->d_jenc + off_fbits);
+    uint8_t* bits = ctx->d_jenc + off_bits;
+    JpegEncChunk ch;
+    int qz[2][64];
+    jpeg_enc_qtables(quality, qz);
+    for (int t = 0; t < 2; ++t)
+        for (int k = 0; k < 64; ++k) ch.qdiv[t][h_jpeg_natural[k]] = (uint16_t)(qz[t][k] << 3);
+    for (int c0 = 0; c0 < B; c0 += JPEG_ENC_CHUNK) {
+        const int n = std::min(JPEG_ENC_CHUNK, B - c0);
+        int64_t max_blocks = 1;
+        for (int i = 0; i < n; ++i) {
+            ch.d[i] = ds[c0 + i];
+            max_blocks = std::max(max_blocks, jpeg_enc_blocks(h[c0 + i], w[c0 + i], hs, vs));
+        }
+        constexpr int bpc = JPEG_ENC_DCT_NT / 8;           // 8x8 blocks per CTA and pass
+        const dim3 gd((unsigned)std::min<int64_t>((max_blocks + bpc - 1) / bpc, 16384), (unsigned)n);
+        jpeg_enc_dct_kernel<<<gd, JPEG_ENC_DCT_NT, 0, st>>>(frames, ch, coef);
+        CU(cudaGetLastError());
+        jpeg_enc_len_kernel<<<n, JPEG_ENC_SCAN_NT, 0, st>>>(ch, coef, offs, fbits, reinterpret_cast<uint32_t*>(bits));
+        CU(cudaGetLastError());
+        const dim3 ge((unsigned)std::min<int64_t>((max_blocks + JPEG_ENC_EMIT_NT - 1) / JPEG_ENC_EMIT_NT, 2048), (unsigned)n);
+        jpeg_enc_emit_kernel<<<ge, JPEG_ENC_EMIT_NT, 0, st>>>(ch, coef, offs, fbits, reinterpret_cast<uint32_t*>(bits));
+        CU(cudaGetLastError());
+        jpeg_enc_stuff_kernel<<<n, JPEG_ENC_STUFF_NT, 0, st>>>(ch, ctx->d_jhdr, fbits, bits, out, len + c0);
+        CU(cudaGetLastError());
+        ctx->launches += 4;
+    }
+    return YF_OK;
+}
+
+extern "C" int yf_encode_jpeg(yf_ctx* ctx, const uint8_t* frames_dev, int B, const int64_t* frame_off, const int32_t* h, const int32_t* w,
+                              int quality, int sampling, uint8_t* out_dev, const int64_t* out_off, int64_t out_bytes, int64_t* len_dev,
+                              void* stream) {
+    CTX_CHECK(ctx);
+    if (!frames_dev || !out_dev || !out_off || !len_dev) { set_err(&ctx->err, "null frames, output, offset or length pointer"); return YF_ERR_ARG; }
+    int hs, vs;
+    int rc = jpeg_enc_params(&ctx->err, quality, sampling, hs, vs);
+    if (rc || (rc = jpeg_enc_check(ctx, B, frame_off, h, w, -1, hs, vs, out_off, out_bytes))) return rc;
+    CU(cudaSetDevice(ctx->device));
+    return jpeg_enc_enqueue(ctx, frames_dev, B, frame_off, h, w, quality, hs, vs, out_dev, out_off, len_dev, (cudaStream_t)stream);
+}
+
+extern "C" int yf_encode_host_jpeg(yf_ctx* ctx, const uint8_t* frames_host, int64_t nbytes, int B, const int64_t* frame_off,
+                                   const int32_t* h, const int32_t* w, int quality, int sampling, uint8_t* out_host, int64_t cap,
+                                   int64_t* len_host, void* stream) {
+    CTX_CHECK(ctx);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!frames_host || !out_host || !len_host) { set_err(&ctx->err, "null frames, output or length pointer"); return YF_ERR_ARG; }
+    int hs, vs;
+    int rc = jpeg_enc_params(&ctx->err, quality, sampling, hs, vs);
+    if (rc || (rc = jpeg_enc_check(ctx, B, frame_off, h, w, nbytes, hs, vs, nullptr, 0))) return rc;
+    std::vector<int64_t> staged(B);                     // each file at its bound on the device, then packed
+    int64_t staged_bytes = 0;
+    for (int b = 0; b < B; ++b) { staged[b] = staged_bytes; staged_bytes += jpeg_enc_file_max(h[b], w[b], hs, vs); }
+    CU(cudaSetDevice(ctx->device));
+    if ((rc = ensure_bgr(ctx, (size_t)nbytes, st))) return rc;
+    if ((rc = jpeg_enc_grow(ctx, &ctx->d_jout, &ctx->jout_cap, (size_t)staged_bytes))) return rc;
+    if ((rc = jpeg_enc_grow(ctx, reinterpret_cast<unsigned char**>(&ctx->d_jlen), &ctx->jlen_cap, sizeof(int64_t) * B))) return rc;
+    CU(cudaMemcpyAsync(ctx->d_bgr, frames_host, (size_t)nbytes, cudaMemcpyHostToDevice, st));      // the frames, one copy
+    if ((rc = jpeg_enc_enqueue(ctx, ctx->d_bgr, B, frame_off, h, w, quality, hs, vs, ctx->d_jout, staged.data(), ctx->d_jlen, st))) return rc;
+    CU(cudaMemcpyAsync(len_host, ctx->d_jlen, sizeof(int64_t) * B, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    int64_t total = 0;
+    for (int b = 0; b < B; ++b) total += len_host[b];
+    if (total > cap) {
+        set_err(&ctx->err, "the %d files take %lld bytes, out_host holds %lld", B, (long long)total, (long long)cap);
+        return YF_ERR_ARG;
+    }
+    if ((rc = jpeg_enc_grow(ctx, &ctx->d_jpack, &ctx->jpack_cap, (size_t)std::max<int64_t>(total, 1)))) return rc;
+    JpegPackChunk pk;
+    int64_t pos = 0, most = 1;
+    for (int c0 = 0; c0 < B; c0 += JPEG_ENC_CHUNK) {
+        const int n = std::min(JPEG_ENC_CHUNK, B - c0);
+        for (int i = 0; i < n; ++i) {
+            pk.src[i] = staged[c0 + i]; pk.dst[i] = pos; pk.len[i] = len_host[c0 + i];
+            pos += pk.len[i];
+            most = std::max(most, pk.len[i]);
+        }
+        const dim3 gp((unsigned)std::min<int64_t>((most + 255) / 256, 1024), (unsigned)n);
+        jpeg_enc_pack_kernel<<<gp, 256, 0, st>>>(pk, ctx->d_jout, ctx->d_jpack);
+        CU(cudaGetLastError());
+        ctx->launches += 1;
+    }
+    CU(cudaMemcpyAsync(out_host, ctx->d_jpack, (size_t)total, cudaMemcpyDeviceToHost, st));       // the files, one copy
+    CU(cudaStreamSynchronize(st));
     return YF_OK;
 }
 
