@@ -297,6 +297,44 @@ int yf_encode_host_jpeg(yf_ctx* ctx, const uint8_t* frames_host, int64_t nbytes,
                         const int32_t* h, const int32_t* w, int quality, int sampling, uint8_t* out_host, int64_t cap,
                         int64_t* len_host, void* stream);
 
+/* ---- YUV 4:2:0 video frames (NV12, I420) on the device -------------------------------------------------------------------- */
+
+/* One 8-bit YUV 4:2:0 frame of h x w pixels, h and w even, every plane at a byte offset from one base pointer. Luma row r is the w bytes
+ * at y_off + r * y_pitch. Chroma sample k (0 <= k < w / 2) of chroma row r (0 <= r < h / 2) is at u_off + r * c_pitch + k * c_step,
+ * and likewise from v_off. Pixel (r, c) takes chroma sample c / 2 of chroma row r / 2.
+ *   NV12 (hardware decoders): c_step = 2, v_off = u_off + 1, the interleaved UV plane after a luma plane of the surface's height.
+ *   I420 (yuv420p, FFmpeg, software decoders): c_step = 1, three separate planes (cv2's [3h/2, w] layout: u_off = h * w,
+ *   v_off = u_off + (h / 2) * (w / 2), c_pitch = w / 2).
+ * 48 bytes (4 bytes of tail padding). */
+typedef struct {
+    int64_t y_off, u_off, v_off;
+    int32_t y_pitch, c_pitch, c_step;
+    int32_t h, w;
+} yf_yuv420;
+
+/* The three YUV entry points check every descriptor before anything is enqueued, and fail with YF_ERR_ARG and a reason that names the
+ * frame: h and w even and in [2, 16384]; y_pitch >= w; c_step >= 1; c_pitch >= (w / 2) * c_step; every byte of every plane inside
+ * [base_dev, base_dev + nbytes); 1 <= B <= max_batch. desc_host is a HOST array of B descriptors. The arithmetic is cv2's for
+ * COLOR_YUV2BGR_NV12 / COLOR_YUV2BGR_I420 (BT.601, limited range, 20-bit fixed point), whatever the layout.
+ *
+ * B frames -> the BGR frames cv2.cvtColor returns, byte for byte, at frame_off[b] of frames_dev ([h, w, 3], contiguous rows: the layout
+ * yf_preprocess_frames reads and yf_encode_jpeg takes; frame_off is a HOST array, every frame inside the frames_bytes of frames_dev).
+ * One launch per 256 frames, enqueued on `stream`. */
+/* Host only, no CUDA: those descriptor checks without a ctx (no max_batch bound); 0, or YF_ERR_ARG with the reason in
+ * yf_last_error(NULL). */
+int yf_yuv420_check(int64_t nbytes, int B, const yf_yuv420* desc_host);
+int yf_yuv420_to_bgr(yf_ctx* ctx, const uint8_t* base_dev, int64_t nbytes, int B, const yf_yuv420* desc_host, uint8_t* frames_dev,
+                     const int64_t* frame_off, int64_t frames_bytes, void* stream);
+/* B frames -> out dev as yf_preprocess_frames writes it for the BGR frames of yf_yuv420_to_bgr ([B, H, W] gray, or [B, 3, H, W] R, G, B
+ * planes for in_ch == 3), byte for byte, without writing the BGR frames anywhere. One launch per 256 frames, enqueued on `stream`. */
+int yf_preprocess_yuv420(yf_ctx* ctx, const uint8_t* base_dev, int64_t nbytes, int B, const yf_yuv420* desc_host, uint8_t* out_dev,
+                         void* stream);
+/* yf_preprocess_yuv420 into the ctx's own input buffer, then yf_detect's forward, decode and NMS: out_dev [B][max_det], counts_dev [B]
+ * and status_dev [B] (may be NULL) as yf_detect writes them, in NETWORK-input coordinates. Enqueued on `stream` without a
+ * synchronisation, after the asynchronous slots in flight. */
+int yf_detect_yuv420(yf_ctx* ctx, const uint8_t* base_dev, int64_t nbytes, int B, const yf_yuv420* desc_host, const yf_post_params* p,
+                     yf_det* out_dev, int32_t* counts_dev, int32_t* status_dev, void* stream);
+
 /* ---- introspection ---------------------------------------------------------------------- */
 
 /* Kernels launched by this ctx since creation (the bench's gpu_launches evidence). */

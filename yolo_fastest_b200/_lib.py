@@ -32,6 +32,17 @@ DET_DTYPE = np.dtype([("x1", "<f8"), ("y1", "<f8"), ("x2", "<f8"), ("y2", "<f8")
 assert DET_DTYPE.itemsize == C.sizeof(YfDet) == 56
 
 
+class YfYuv420(C.Structure):
+    """yf_yuv420: one YUV 4:2:0 frame, planes at byte offsets from one base pointer (48 bytes with its tail padding)."""
+    _fields_ = [("y_off", C.c_int64), ("u_off", C.c_int64), ("v_off", C.c_int64),
+                ("y_pitch", C.c_int32), ("c_pitch", C.c_int32), ("c_step", C.c_int32), ("h", C.c_int32), ("w", C.c_int32)]
+
+
+YUV_DTYPE = np.dtype([("y_off", "<i8"), ("u_off", "<i8"), ("v_off", "<i8"), ("y_pitch", "<i4"), ("c_pitch", "<i4"),
+                      ("c_step", "<i4"), ("h", "<i4"), ("w", "<i4")], align=True)
+assert YUV_DTYPE.itemsize == C.sizeof(YfYuv420) == 48
+
+
 class YfPostParams(C.Structure):
     _fields_ = [("anchors", C.c_double * 2 * YF_MAX_ANCHORS * 2),
                 ("conf_thres", C.c_double), ("nms_thres", C.c_double),
@@ -74,6 +85,10 @@ SYMBOLS = [
     ("yf_jpeg_encode_header", C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int64]),
     ("yf_encode_jpeg", C.c_int, [_P, _P, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, _P, C.c_int64, _P, _P]),
     ("yf_encode_host_jpeg", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.c_int, C.c_int, _P, C.c_int64, _P, _P]),
+    ("yf_yuv420_check", C.c_int, [C.c_int64, C.c_int, _P]),
+    ("yf_yuv420_to_bgr", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P, C.c_int64, _P]),
+    ("yf_preprocess_yuv420", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, _P, _P]),
+    ("yf_detect_yuv420", C.c_int, [_P, _P, C.c_int64, C.c_int, _P, C.POINTER(YfPostParams), _P, _P, _P, _P]),
     ("yf_compact_dets", C.c_int, [_P, _P, _P, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P]),
     ("yf_launch_count", C.c_int64, [_P]),
     ("yf_profile_forward", C.c_int, [_P, _P, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_float), C.c_int]),

@@ -28,6 +28,7 @@
 #include "yf_prep.cuh"
 #include "yf_jpeg.cuh"
 #include "yf_jpeg_enc.cuh"
+#include "yf_yuv.cuh"
 
 using namespace yf;
 
@@ -1461,6 +1462,8 @@ extern "C" int yf_create_variant(yf_ctx** out, int device, int in_ch, int num_cl
         cudaFuncSetAttribute(post_kernel<POST_SRC_ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 12),
         cudaFuncSetAttribute(prep_frames_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
         cudaFuncSetAttribute(prep_frames_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
+        cudaFuncSetAttribute(prep_yuv_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
+        cudaFuncSetAttribute(prep_yuv_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, PREP_SMEM_CAP),
         cudaFuncSetAttribute(jpeg_entropy_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, JPEG_TABS_BYTES),
         cudaFuncSetAttribute(jpeg_entropy_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * JPEG_TABS_BYTES),
         init_irb<CfgRes2>(), init_irb<CfgDown2>(), init_irb<CfgRes3a>(), init_irb<CfgWide3>(),
@@ -2435,6 +2438,127 @@ extern "C" int yf_encode_host_jpeg(yf_ctx* ctx, const uint8_t* frames_host, int6
     CU(cudaMemcpyAsync(out_host, ctx->d_jpack, (size_t)total, cudaMemcpyDeviceToHost, st));       // the files, one copy
     CU(cudaStreamSynchronize(st));
     return YF_OK;
+}
+
+// ---- YUV 4:2:0 frames (yf_yuv.cuh): every descriptor checked on the host, one launch per chunk of 256 frames --------------------
+// every descriptor against the size rules and the buffer; err == NULL: the global message of yf_last_error(NULL)
+static int yuv_desc_check(std::string* err, int64_t nbytes, int B, const yf_yuv420* d) {
+    if (!d) { set_err(err, "null descriptor array"); return YF_ERR_ARG; }
+    for (int b = 0; b < B; ++b) {
+        const yf_yuv420& f = d[b];
+        if (f.h < 2 || f.w < 2 || f.h > kPrepMaxSide || f.w > kPrepMaxSide || (f.h & 1) || (f.w & 1)) {
+            set_err(err, "frame %d: size %dx%d: YUV 4:2:0 sizes are even and in [2, %d]", b, f.h, f.w, kPrepMaxSide); return YF_ERR_ARG;
+        }
+        if (f.y_pitch < f.w) { set_err(err, "frame %d: luma pitch %d below the width %d", b, f.y_pitch, f.w); return YF_ERR_ARG; }
+        if (f.c_step < 1) { set_err(err, "frame %d: chroma step %d below 1", b, f.c_step); return YF_ERR_ARG; }
+        if ((int64_t)f.c_pitch < (int64_t)(f.w / 2) * f.c_step) {
+            set_err(err, "frame %d: chroma pitch %d below %d samples of step %d", b, f.c_pitch, f.w / 2, f.c_step); return YF_ERR_ARG;
+        }
+        const int64_t cspan = (int64_t)(f.h / 2 - 1) * f.c_pitch + (int64_t)(f.w / 2 - 1) * f.c_step + 1;
+        const struct { const char* name; int64_t off, span; } planes[3] = {
+            {"luma", f.y_off, (int64_t)(f.h - 1) * f.y_pitch + f.w}, {"U", f.u_off, cspan}, {"V", f.v_off, cspan}};
+        for (const auto& pl : planes) {
+            if (pl.off < 0 || pl.off > nbytes - pl.span) {
+                set_err(err, "frame %d: %s plane bytes [%lld, %lld) outside the %lld-byte buffer", b, pl.name, (long long)pl.off,
+                        (long long)(pl.off + pl.span), (long long)nbytes);
+                return YF_ERR_ARG;
+            }
+        }
+    }
+    return YF_OK;
+}
+
+extern "C" int yf_yuv420_check(int64_t nbytes, int B, const yf_yuv420* desc_host) {
+    if (B < 1) { set_err(nullptr, "batch %d < 1", B); return YF_ERR_ARG; }
+    return yuv_desc_check(nullptr, nbytes, B, desc_host);
+}
+
+static int yuv_check(yf_ctx* ctx, const uint8_t* base, int64_t nbytes, int B, const yf_yuv420* d) {
+    if (!base) { set_err(&ctx->err, "null base pointer"); return YF_ERR_ARG; }
+    if (B < 1 || B > ctx->max_batch) { set_err(&ctx->err, "batch %d outside [1, max_batch=%d]", B, ctx->max_batch); return YF_ERR_ARG; }
+    return yuv_desc_check(&ctx->err, nbytes, B, d);
+}
+
+extern "C" int yf_yuv420_to_bgr(yf_ctx* ctx, const uint8_t* base_dev, int64_t nbytes, int B, const yf_yuv420* desc_host, uint8_t* frames_dev,
+                                const int64_t* frame_off, int64_t frames_bytes, void* stream) {
+    CTX_CHECK(ctx);
+    if (!frames_dev || !frame_off) { set_err(&ctx->err, "null frames or frame offset pointer"); return YF_ERR_ARG; }
+    int rc = yuv_check(ctx, base_dev, nbytes, B, desc_host);
+    if (rc) return rc;
+    for (int b = 0; b < B; ++b) {
+        const int64_t size = (int64_t)desc_host[b].h * desc_host[b].w * 3;
+        if (frame_off[b] < 0 || frame_off[b] > frames_bytes - size) {
+            set_err(&ctx->err, "frame %d: BGR bytes [%lld, %lld) outside the %lld-byte frame buffer", b, (long long)frame_off[b],
+                    (long long)(frame_off[b] + size), (long long)frames_bytes);
+            return YF_ERR_ARG;
+        }
+    }
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    YuvBgrFrames ch;
+    for (int c0 = 0; c0 < B; c0 += YUV_CHUNK) {
+        const int n = std::min(YUV_CHUNK, B - c0);
+        long long most = 1;
+        for (int i = 0; i < n; ++i) {
+            ch.f[i] = desc_host[c0 + i];
+            ch.dst[i] = frame_off[c0 + i];
+            most = std::max(most, (long long)(ch.f[i].h / 2) * ((ch.f[i].w + 3) / 4));
+        }
+        const dim3 grid((unsigned)std::min<long long>((most + YUV_NT - 1) / YUV_NT, 1024), (unsigned)n);
+        yuv_bgr_kernel<<<grid, YUV_NT, 0, st>>>(base_dev, ch, frames_dev);
+        CU(cudaGetLastError());
+        ctx->launches += 1;
+    }
+    return YF_OK;
+}
+
+// descriptors already checked -> out [B, in_ch, H, W]; prep_yuv_kernel with frames_enqueue's launch shape
+static int yuv_prep_enqueue(yf_ctx* ctx, const uint8_t* base, int B, const yf_yuv420* d, uint8_t* out, cudaStream_t st) {
+    const int nsm = ctx->groups.empty() ? 148 : ctx->groups[0].a.nsm;
+    const long long groups = (ctx->H + PREP_R - 1) / PREP_R;
+    const size_t per_img = (size_t)ctx->in_ch * ctx->H * ctx->W;
+    YuvFrames fr;
+    for (int c0 = 0; c0 < B; c0 += YUV_CHUNK) {
+        const int n = std::min(YUV_CHUNK, B - c0);
+        int smem = 0;                                   // from the widest frame of the chunk that is staged
+        for (int i = 0; i < n; ++i) {
+            fr.f[i] = d[c0 + i];
+            if (yuv_stageable(base, fr.f[i], ctx->in_ch, PREP_SMEM_CAP)) smem = std::max(smem, prep_stage_bytes(fr.f[i].w, ctx->in_ch));
+        }
+        auto kern = ctx->in_ch == 1 ? prep_yuv_kernel<1> : prep_yuv_kernel<3>;
+        int per_sm = 1;
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, PREP_NT, smem));
+        const int grid = (int)std::min<long long>((long long)n * groups, (long long)nsm * std::max(per_sm, 1));
+        kern<<<grid, PREP_NT, smem, st>>>(base, fr, n, out + c0 * per_img, ctx->H, ctx->W, smem);
+        CU(cudaGetLastError());
+        ctx->launches += 1;
+    }
+    return YF_OK;
+}
+
+extern "C" int yf_preprocess_yuv420(yf_ctx* ctx, const uint8_t* base_dev, int64_t nbytes, int B, const yf_yuv420* desc_host, uint8_t* out_dev,
+                                    void* stream) {
+    CTX_CHECK(ctx);
+    if (!out_dev) { set_err(&ctx->err, "null output pointer"); return YF_ERR_ARG; }
+    int rc = yuv_check(ctx, base_dev, nbytes, B, desc_host);
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    return yuv_prep_enqueue(ctx, base_dev, B, desc_host, out_dev, (cudaStream_t)stream);
+}
+
+extern "C" int yf_detect_yuv420(yf_ctx* ctx, const uint8_t* base_dev, int64_t nbytes, int B, const yf_yuv420* desc_host, const yf_post_params* p,
+                                yf_det* out_dev, int32_t* counts_dev, int32_t* status_dev, void* stream) {
+    CTX_CHECK(ctx);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!p || !out_dev || !counts_dev) { set_err(&ctx->err, "null argument"); return YF_ERR_ARG; }
+    if (p->max_det < 1) { set_err(&ctx->err, "max_det must be >= 1"); return YF_ERR_ARG; }
+    int rc = yuv_check(ctx, base_dev, nbytes, B, desc_host);
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    if (!ctx->weights_loaded) { set_err(&ctx->err, "yf_load_weights has not been called"); return YF_ERR_STATE; }
+    ORDER(ctx, st);
+    if ((rc = yuv_prep_enqueue(ctx, base_dev, B, desc_host, ctx->d_u8, st))) return rc;
+    return detect_fixed(ctx, ctx->d_u8, true, B, p, out_dev, counts_dev, status_dev, st);
 }
 
 // ---- asynchronous, double-buffered host path --------------------------------------------------------------

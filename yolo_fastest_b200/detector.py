@@ -292,6 +292,130 @@ def pack_frames(frames, dst, off):
         dst[int(o):int(o) + a.size].reshape(a.shape)[...] = a
 
 
+YUV_FORMATS = ("nv12", "i420")
+
+
+def _yuv_plane(t, b, what, rows, cols):
+    """A cuda uint8 plane tensor [rows, cols] with unit column stride -> (address, row pitch, end address)."""
+    if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype == torch.uint8 and t.dim() == 2):
+        raise _lib.YfError("frame %d: the %s plane is not a 2-D cuda uint8 tensor" % (b, what))
+    if list(t.shape) != [rows, cols]:
+        raise _lib.YfError("frame %d: the %s plane is %s, expected [%d, %d]" % (b, what, list(t.shape), rows, cols))
+    if t.stride(1) != 1 or t.stride(0) < cols:
+        raise _lib.YfError("frame %d: the %s plane has strides %s: columns must be adjacent and rows must not overlap" % (b, what, t.stride()))
+    p = t.data_ptr()
+    return p, t.stride(0), p + (rows - 1) * t.stride(0) + cols
+
+
+def yuv_layout(frames, fmt="nv12"):
+    """Check a list of YUV 4:2:0 frames and describe them -> (desc, on_dev, base, nbytes), desc a YUV_DTYPE array of yf_yuv420.
+
+    A frame is cv2's form, a 2-D uint8 [3h / 2, w] numpy array or tensor (I420: contiguous; cuda NV12: unit column stride, any row
+    stride), or, on the device only, a tuple of plane tensors: (Y [h, w], UV [h / 2, w]) for nv12, (Y, U [h / 2, w / 2],
+    V [h / 2, w / 2]) for i420 (U and V with one row pitch), each plane with its own pitch and allocation. Cuda frames are described
+    in place, with offsets from the lowest plane address `base` and `nbytes` up to the highest plane end. Host frames are described
+    as pack_yuv lays them out (base = None): back to back, each at a multiple of FRAME_ALIGN, in cv2's contiguous layout.
+    Raises YfError naming the first frame that does not fit."""
+    if fmt not in YUV_FORMATS:
+        raise _lib.YfError("fmt %r: YUV frames are %s" % (fmt, " or ".join(repr(f) for f in YUV_FORMATS)))
+    if not isinstance(frames, (list, tuple)) or len(frames) == 0:
+        raise _lib.YfError("frames: a non-empty list of YUV 4:2:0 frames")
+    nv12 = fmt == "nv12"
+    B = len(frames)
+    desc = np.zeros(B, _lib.YUV_DTYPE)
+    on_dev = [isinstance(f, tuple) or (isinstance(f, torch.Tensor) and f.is_cuda) for f in frames]
+    if any(on_dev) and not all(on_dev):
+        raise _lib.YfError("frames must be all on the host or all on the device")
+    dev = all(on_dev)
+    lo, hi, pos, ptrs = None, 0, 0, []
+    for b, f in enumerate(frames):
+        if isinstance(f, tuple):
+            if len(f) != (2 if nv12 else 3) or not isinstance(f[0], torch.Tensor) or f[0].dim() != 2:
+                raise _lib.YfError("frame %d: a %s plane tuple is %s" % (b, fmt, "(Y, UV)" if nv12 else "(Y, U, V)"))
+            h, w = int(f[0].shape[0]), int(f[0].shape[1])
+        else:
+            if not isinstance(f, (np.ndarray, torch.Tensor)):
+                raise _lib.YfError("frame %d is a %s, not a numpy array, tensor or tuple of plane tensors" % (b, type(f).__name__))
+            if f.dtype != (torch.uint8 if isinstance(f, torch.Tensor) else np.uint8):
+                raise _lib.YfError("frame %d is %s, frames are uint8" % (b, f.dtype))
+            if f.ndim != 2 or f.shape[0] % 3:
+                raise _lib.YfError("frame %d has shape %s, a %s frame in cv2's form is [3h / 2, w]" % (b, tuple(f.shape), fmt))
+            h, w = int(f.shape[0]) * 2 // 3, int(f.shape[1])
+        if h % 2 or w % 2 or not (2 <= h <= MAX_FRAME_SIDE and 2 <= w <= MAX_FRAME_SIDE):
+            raise _lib.YfError("frame %d is %dx%d: YUV 4:2:0 sizes are even and in [2, %d]" % (b, h, w, MAX_FRAME_SIDE))
+        d = desc[b]
+        d["h"], d["w"] = h, w
+        if isinstance(f, tuple):
+            py, d["y_pitch"], ey = _yuv_plane(f[0], b, "Y", h, w)
+            if nv12:
+                pu, d["c_pitch"], eu = _yuv_plane(f[1], b, "UV", h // 2, w)
+                pv, ev = pu + 1, eu
+            else:
+                pu, d["c_pitch"], eu = _yuv_plane(f[1], b, "U", h // 2, w // 2)
+                pv, vp, ev = _yuv_plane(f[2], b, "V", h // 2, w // 2)
+                if vp != d["c_pitch"]:
+                    raise _lib.YfError("frame %d: the U and V planes have pitches %d and %d, they must share one" % (b, d["c_pitch"], vp))
+            ptrs.append((py, pu, pv))
+            lo = min(x for x in (lo, py, pu, pv) if x is not None)
+            hi = max(hi, ey, eu, ev)
+        else:
+            contiguous = f.is_contiguous() if isinstance(f, torch.Tensor) else f.flags["C_CONTIGUOUS"]
+            if not nv12 and not contiguous:
+                raise _lib.YfError("frame %d: an i420 frame in cv2's form must be contiguous (cv2 reads the chroma of a row-padded i420 array "
+                                   "as two rows per stride); pass its planes as a tuple" % b)
+            if dev:
+                if f.stride(1) != 1:
+                    raise _lib.YfError("frame %d has strides %s: columns must be adjacent" % (b, f.stride()))
+                p, pitch = f.data_ptr(), f.stride(0)
+                ptrs.append((p, p + h * pitch, None))
+                lo = p if lo is None else min(lo, p)
+                hi = max(hi, p + (h * 3 // 2 - 1) * pitch + w)
+            else:
+                p, pitch = pos, w
+                pos += -(-h * 3 // 2 * w // FRAME_ALIGN) * FRAME_ALIGN
+            d["y_off"], d["y_pitch"] = p, pitch
+            if nv12:
+                d["u_off"], d["v_off"], d["c_pitch"] = p + h * pitch, p + h * pitch + 1, pitch
+            else:
+                d["u_off"], d["v_off"], d["c_pitch"] = p + h * w, p + h * w + (h // 2) * (w // 2), w // 2
+        d["c_step"] = 2 if nv12 else 1
+    if dev:
+        for d, (py, pu, pv) in zip(desc, ptrs):
+            d["y_off"] = py - lo
+            if pv is not None:                          # planes of a tuple
+                d["u_off"], d["v_off"] = pu - lo, pv - lo
+            else:                                       # cv2's form: offsets were relative to the frame's own address
+                d["u_off"], d["v_off"] = d["u_off"] - py + d["y_off"], d["v_off"] - py + d["y_off"]
+        nbytes = hi - lo
+    else:
+        nbytes = int(desc[-1]["y_off"]) + int(desc[-1]["h"]) * 3 // 2 * int(desc[-1]["w"])
+    if _lib.lib().yf_yuv420_check(nbytes, B, desc.ctypes.data) != 0:       # the library's own checks, before anything is enqueued
+        raise _lib.YfError(_lib.lib().yf_last_error(None).decode())
+    return desc, dev, lo if dev else None, nbytes
+
+
+def pack_yuv(frames, dst, desc):
+    """Copy host frames in cv2's form into the uint8 numpy buffer `dst` at the offsets yuv_layout gave them (any strides)."""
+    for f, d in zip(frames, desc):
+        a = f.numpy() if isinstance(f, torch.Tensor) else f
+        o = int(d["y_off"])
+        dst[o:o + a.size].reshape(a.shape)[...] = a
+
+
+def _to_frame_coords(rows, Ho, Wo, H, W):
+    """adjust_coord's arithmetic with each frame's own size, in place: round(v * (h / H)), round(v * (w / W)) (detect.py:131-139)."""
+    for rr, h, w in zip(rows, Ho, Wo):
+        if [int(h), int(w)] == [H, W]:
+            continue
+        scale_h, scale_w = int(h) / H, int(w) / W
+        for r in rr:
+            r[0] = round(r[0] * scale_w)
+            r[2] = round(r[2] * scale_w)
+            r[1] = round(r[1] * scale_h)
+            r[3] = round(r[3] * scale_h)
+    return rows
+
+
 class Detect_YOLO:
     def __init__(self, device, model_path, config_params, logger):
         device = torch.device(device)
@@ -317,6 +441,7 @@ class Detect_YOLO:
         self._slots = {}
         self._frames_pin = None        # grow-only pinned staging of packed host frames (pre_process_frames / detect_frames)
         self._frames_ev = None         # end of the last asynchronous copy out of it
+        self._yuv_res = (None,)        # ((B, max_det), out, counts, status): detect_yuv's device result buffers
 
     # ---- host-side image handling (unchanged semantics, detect.py:107-139) ------------------------
     def _load_gray(self, img_path):
@@ -472,17 +597,7 @@ class Detect_YOLO:
         if raw:
             return res
         rows = [_rows_from_dets(d) for d in res]
-        if adjust:
-            for rr, h, w in zip(rows, Ho, Wo):
-                if [int(h), int(w)] == [H, W]:
-                    continue
-                scale_h, scale_w = int(h) / H, int(w) / W
-                for r in rr:
-                    r[0] = round(r[0] * scale_w)
-                    r[2] = round(r[2] * scale_w)
-                    r[1] = round(r[1] * scale_h)
-                    r[3] = round(r[3] * scale_h)
-        return rows
+        return _to_frame_coords(rows, Ho, Wo, H, W) if adjust else rows
 
     # ---- JPEG files decoded on the device (yf_decode_jpeg / yf_detect_host_jpeg) ---------------------------------------------------
     def decode_jpeg(self, files):
@@ -518,16 +633,7 @@ class Detect_YOLO:
         if not raw:
             rows = [_rows_from_dets(d) for d in rows]
             if adjust:
-                H, W = self.input_shape[0:2]
-                for rr, h, w in zip(rows, Ho, Wo):
-                    if [int(h), int(w)] == [H, W]:
-                        continue
-                    scale_h, scale_w = int(h) / H, int(w) / W
-                    for r in rr:
-                        r[0] = round(r[0] * scale_w)
-                        r[2] = round(r[2] * scale_w)
-                        r[1] = round(r[1] * scale_h)
-                        r[3] = round(r[3] * scale_h)
+                _to_frame_coords(rows, Ho, Wo, *self.input_shape[0:2])
         return (rows, frames) if return_frames else rows
 
     def _detect_jpeg(self, files_u8, off, ln, foff, Ho, Wo, fbytes, max_det, want_frames):
@@ -597,6 +703,84 @@ class Detect_YOLO:
                                                          ln.ctypes.data, C.c_void_p(stream)), ctx.handle)
         ends = np.cumsum(ln)
         return [packed[int(e - n):int(e)].tobytes() for e, n in zip(ends, ln)]
+
+    # ---- YUV 4:2:0 video frames (yf_yuv420_to_bgr / yf_preprocess_yuv420 / yf_detect_yuv420) --------------------------------------
+    def _yuv_on_device(self, frames, fmt):
+        """yuv_layout, and host frames packed into the pinned staging and copied up once -> (desc, base address, nbytes, staging)."""
+        desc, on_dev, base, nbytes = yuv_layout(frames, fmt)
+        if on_dev:
+            for b, f in enumerate(frames):
+                for t in (f if isinstance(f, tuple) else (f,)):
+                    if t.device != self.device:
+                        raise _lib.YfError("frame %d is on %s, the detector on %s" % (b, t.device, self.device))
+            return desc, base, nbytes, None
+        pin = self._frames_pinned(nbytes)
+        pack_yuv(frames, pin.numpy(), desc)
+        staged = torch.empty((nbytes,), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device)
+            staged.copy_(pin[:nbytes], non_blocking=True)
+            self._frames_ev = torch.cuda.Event()
+            self._frames_ev.record(stream)
+        return desc, staged.data_ptr(), nbytes, staged
+
+    def yuv_to_bgr(self, frames, fmt="nv12"):
+        """YUV 4:2:0 frames (see yuv_layout: cv2's [3h / 2, w] form, host or cuda, or cuda plane tuples) -> list of cuda uint8
+        [h, w, 3] BGR tensors, each byte for byte cv2.cvtColor(frame, COLOR_YUV2BGR_NV12 / COLOR_YUV2BGR_I420). fmt is "nv12" or
+        "i420". The frames share one buffer, in the layout pre_process_frames and encode_jpeg take. Enqueued on the current stream."""
+        desc, base, nbytes, staged = self._yuv_on_device(frames, fmt)
+        B = len(desc)
+        sizes = desc["h"].astype(np.int64) * desc["w"] * 3
+        foff = np.concatenate([[0], np.cumsum(-(-sizes // FRAME_ALIGN) * FRAME_ALIGN)[:-1]]).astype(np.int64)
+        out = torch.empty((int(foff[-1] + sizes[-1]),), dtype=torch.uint8, device=self.device)
+        ctx = self.model.context(self.device, self.input_shape[0], self.input_shape[1], B)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            _lib.check(_lib.lib().yf_yuv420_to_bgr(ctx.handle, base, nbytes, B, desc.ctypes.data, out.data_ptr(), foff.ctypes.data,
+                                                  out.numel(), C.c_void_p(stream)), ctx.handle)
+        return [out[int(o):int(o) + int(s)].view(int(d["h"]), int(d["w"]), 3) for o, s, d in zip(foff, sizes, desc)]
+
+    def pre_process_yuv(self, frames, fmt="nv12"):
+        """YUV 4:2:0 frames (as yuv_to_bgr) -> the cuda uint8 network input pre_process_frames returns for their BGR frames, byte for
+        byte ([B, H, W] gray, or [B, 3, H, W] R, G, B planes), in one fused kernel launch per 256 frames: no BGR frame is written."""
+        desc, base, nbytes, staged = self._yuv_on_device(frames, fmt)
+        B = len(desc)
+        H, W, chans = self.input_shape[0:3]
+        ctx = self.model.context(self.device, H, W, B)
+        out = torch.empty((B, H, W) if chans == 1 else (B, chans, H, W), dtype=torch.uint8, device=self.device)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            _lib.check(_lib.lib().yf_preprocess_yuv420(ctx.handle, base, nbytes, B, desc.ctypes.data, out.data_ptr(), C.c_void_p(stream)),
+                       ctx.handle)
+        return out
+
+    def detect_yuv(self, frames, fmt="nv12", max_det=64, raw=False, adjust=True):
+        """YUV 4:2:0 frames (as yuv_to_bgr) -> the rows detect_frames returns for their BGR frames: one yf_detect_yuv420 call (fused
+        pre-processing into the context's input buffer, forward, decode, NMS), the results back once. Cuda frames are read in place;
+        host frames travel in one copy. adjust as in detect_frames. Bad input raises YfError naming the frame before any launch."""
+        desc, base, nbytes, staged = self._yuv_on_device(frames, fmt)
+        res = self._detect_yuv(desc, base, nbytes, max_det)
+        if raw:
+            return res
+        rows = [_rows_from_dets(d) for d in res]
+        return _to_frame_coords(rows, desc["h"], desc["w"], *self.input_shape[0:2]) if adjust else rows
+
+    def _detect_yuv(self, desc, base, nbytes, max_det):
+        B = len(desc)
+        H, W = self.input_shape[0:2]
+        ctx = self.model.context(self.device, H, W, B)
+        key = (B, max_det)
+        if self._yuv_res[0] != key:     # the same result buffers call after call, so small batches replay one CUDA graph
+            self._yuv_res = (key, torch.empty((B, max_det, _lib.DET_DTYPE.itemsize), dtype=torch.uint8, device=self.device),
+                             torch.empty((B,), dtype=torch.int32, device=self.device), torch.empty((B,), dtype=torch.int32, device=self.device))
+        _, out, cnt, st = self._yuv_res
+        p = self.post_process._params(_lib.MODE_DETECT, max_det)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream(self.device).cuda_stream
+            _lib.check(_lib.lib().yf_detect_yuv420(ctx.handle, base, nbytes, B, desc.ctypes.data, C.byref(p), out.data_ptr(), cnt.data_ptr(),
+                                                  st.data_ptr(), C.c_void_p(stream)), ctx.handle)
+            h_out, h_cnt, h_st = out.cpu(), cnt.cpu(), st.cpu()
+        return _finish(h_out, h_cnt, h_st, B, max_det, lambda need: self._detect_yuv(desc, base, nbytes, need))
 
     # ---- batched detection through the C ABI with host buffers -----------------------------------------
     def detect_batch(self, u8_batch, max_det=64, raw=False):
